@@ -18,6 +18,9 @@ wavefront fill) -- BASELINE configs[4]; the throughput of a stream of alignments
 
     python bench.py --workload reads [--pairs 10000000]    BASELINE configs[3]: batched reads x windows
 
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float64; float32 for per-pair
+scores, at most 64 MB in all), so that two builds can be compared output for output on the same seeded inputs.
+
   value     whole-job GCUPS, sequences resident in HBM, device time (CUDA events
             recorded by the library on the stream it launches on), max over ranks
   e2e       same metric through the C ABI with HOST buffers (H2D + D2H inside)
@@ -72,6 +75,24 @@ def emit(obj):
     out = _JSON_OUT if _JSON_OUT is not None else sys.stdout
     out.write(json.dumps(obj) + "\n")
     out.flush()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_MAX_PAIRS = 2_000_000     # --workload reads: 2 schemes x 4 B + an 8 B index per pair = 32 MB
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: one <name>.npy per array (float32 / float64 only)"""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log(f"bench.py: wrote {', '.join(sorted(arrays))} to {directory}")
+
+
+def result_arrays(score, end_i, end_j):
+    return {"score": np.array([score], dtype=np.float64), "end_cell": np.array([end_i, end_j], dtype=np.float64)}
 
 
 class ClockSampler:
@@ -147,9 +168,11 @@ def run_reference(args, rank):
     side = int(args.cpu_sample) or 150000
     times = []
     for i in range(args.warmup + args.steps):
-        g, dt, _ = cpu_baseline(q, s, side, side, threads)
+        g, dt, sc = cpu_baseline(q, s, side, side, threads)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result_arrays(*sc))
     ms = 1e3 * float(np.mean(times))
     val = side * side / (ms * 1e-3) / 1e9
     sample = f"first {side} x {side} cells of the workload per step ({side*side:.3g} cells), all {threads} host threads"
@@ -243,6 +266,13 @@ def run_reads(args, rank, world, local_rank):
         torch.cuda.synchronize()
         return al.score_batch_packed2(mode, pb_dev, d_sc.data_ptr(), scoring, device=True)
 
+    # --dump-outputs: the scores of a fixed, seeded sample of the pairs (all of them up to DUMP_MAX_PAIRS)
+    dumped = {}
+    if args.dump_outputs:
+        pick = np.arange(npairs) if npairs <= DUMP_MAX_PAIRS else \
+            np.sort(np.random.default_rng(0).choice(npairs, DUMP_MAX_PAIRS, replace=False))
+        mine_pick = torch.from_numpy(pick[(pick >= p0) & (pick < p1)] - p0).cuda()
+
     results = {}
     sampler = ClockSampler(local_rank)
     for mi, mode in enumerate(modes):
@@ -257,6 +287,13 @@ def run_reads(args, rank, world, local_rank):
             ms += r.kernel_ms
             nl += r.kernel_launches
         barrier()
+        if args.dump_outputs:
+            got = d_sc[mine_pick].float().cpu().numpy()        # |score| < 2**24: exact in float32
+            if dist is not None:
+                parts = [None] * world
+                dist.all_gather_object(parts, got)
+                got = np.concatenate(parts)                     # ranks hold contiguous, ascending pair ranges
+            dumped[f"scores_{mode}"] = got
         chk = int(d_sc.to(torch.int64).sum().item())          # 64-bit checksum of this rank's scores
         # e2e: pinned host arrays through the C ABI
         e2e_steps = max(1, min(args.steps, 3))
@@ -283,6 +320,8 @@ def run_reads(args, rank, world, local_rank):
         if dist is not None:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**dumped, "pair_index": pick.astype(np.float64)})
     # oracle check on the first pairs of rank 0 (both schemes) + CPU baseline timing of the same sample
     from oracle import oracle as O
     sq, ss = sample
@@ -349,7 +388,11 @@ def main():
                     help="N > 1, 'stream' leg: consecutive alignments relaxed side by side in one launch per rank")
     ap.add_argument("--stream-steps", type=int, default=-1,
                     help="N > 1: alignments of the streamed leg (default: 2 launches of --pairs-per-launch; 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32/float64, <= 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     _claim_stdout()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -513,6 +556,8 @@ def main():
         if dist is not None:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result_arrays(res.score, res.end_i, res.end_j))
 
     # ---- parity inside the bench: the frozen CPU result of the FULL-SIZE workload, and the CPU sample scored on the GPU
     gold = golden_c2() if args.scale == 1.0 else None
