@@ -224,13 +224,21 @@ class Aligner:
         return ops.value, mhz.value
 
 
-def plan_launch(mode, lenq: int, lens: int, affine: bool = False, sm_count: int = 148, chained: bool = False) -> dict:
+def plan_launch(mode, lenq: int, lens: int, affine: bool = False, sm_count: int = 148, chained: bool = False,
+                scheme=None) -> dict:
     """The launch the engine makes for one lenq x lens score-only problem (``anyseq_plan_launch``): strip width, tile
-    height, cell form, bands, grid.  Host logic only -- works without a GPU."""
+    height, cell form, bands, grid, packed cells.  Host logic only -- works without a GPU.  ``scheme`` = (same, diff,
+    gap_init, gap_extend) (``anyseq_plan_launch_scheme``; it decides packed_cells, and gap_init != 0 means affine);
+    default: (2, -1, -2, -1), or (2, -1, 0, -1) with affine=False."""
     L = capi.load_library()
     plan = capi.LaunchPlan()
     m = capi.MODES[mode] if isinstance(mode, str) else int(mode)
-    rc = L.anyseq_plan_launch(int(sm_count), m, int(bool(affine)), int(lenq), int(lens), int(bool(chained)), C.byref(plan))
+    if scheme is None:
+        rc = L.anyseq_plan_launch(int(sm_count), m, int(bool(affine)), int(lenq), int(lens), int(bool(chained)), C.byref(plan))
+    else:
+        same, diff, gap_init, gap_extend = (int(v) for v in scheme)
+        sc = capi.Scoring(m, same, diff, gap_init, gap_extend)
+        rc = L.anyseq_plan_launch_scheme(int(sm_count), C.byref(sc), int(lenq), int(lens), int(bool(chained)), C.byref(plan))
     if rc != 0:
         raise AnyseqError(rc, L.anyseq_last_error().decode())
     return {name: int(getattr(plan, name)) for name, _ in capi.LaunchPlan._fields_}

@@ -32,7 +32,7 @@ EXPORTED_SYMBOLS = [
     "anyseq_batch_stream_collect", "anyseq_batch_stream_release", "anyseq_batch_stream_stats", "anyseq_batch_stream_close",
     "anyseq_strip_inbox_create", "anyseq_strip_inbox_open", "anyseq_strip_inbox_reset",
     "anyseq_strip_inbox_destroy", "anyseq_score_strip_device", "anyseq_score_strip", "anyseq_score_strip_device_multi", "anyseq_strip_combine",
-    "anyseq_measure_int_peak", "anyseq_device_info", "anyseq_plan_launch",
+    "anyseq_measure_int_peak", "anyseq_device_info", "anyseq_plan_launch", "anyseq_plan_launch_scheme",
 ]
 
 
@@ -49,7 +49,7 @@ class Result(C.Structure):
 class LaunchPlan(C.Structure):
     _fields_ = [("cols_per_lane", C.c_int32), ("rows_per_step", C.c_int32), ("cell_form", C.c_int32), ("strips", C.c_int32),
                 ("warps_per_scheduler", C.c_int32), ("bands", C.c_int32), ("band_rows", C.c_int32), ("grid", C.c_int32),
-                ("warps_per_cta", C.c_int32), ("first_items", C.c_int64)]
+                ("warps_per_cta", C.c_int32), ("first_items", C.c_int64), ("packed_cells", C.c_int32)]
 
 
 class StripPartial(C.Structure):
@@ -188,6 +188,8 @@ def load_library(path: str | None = None):
     L.anyseq_device_info.argtypes = [vp, C.POINTER(C.c_int), C.POINTER(C.c_int), vp]
     L.anyseq_plan_launch.restype = C.c_int
     L.anyseq_plan_launch.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(LaunchPlan)]
+    L.anyseq_plan_launch_scheme.restype = C.c_int
+    L.anyseq_plan_launch_scheme.argtypes = [C.c_int, C.POINTER(Scoring), C.c_int, C.c_int, C.c_int, C.POINTER(LaunchPlan)]
     if path is None:
         _lib = L
     return L

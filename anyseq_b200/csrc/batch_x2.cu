@@ -19,10 +19,6 @@ namespace anyseq {
 
 constexpr int kNeg16 = -30000;     // "minus infinity" of E / F in a signed 16-bit half
 
-__device__ __forceinline__ unsigned pack2(int lo, int hi) { return ((unsigned)lo & 0xffffu) | ((unsigned)hi << 16); }
-__device__ __forceinline__ int lo16(unsigned v) { return (int)(short)(v & 0xffffu); }
-__device__ __forceinline__ int hi16(unsigned v) { return (int)(short)(v >> 16); }
-
 struct X2Const {
     int one;
     unsigned ge2;        // (ge, ge) as 16-bit fields (DPX operand)
@@ -32,19 +28,6 @@ struct X2Const {
     int dhi;             // (same - diff) << 16
     unsigned floor2;     // local: (bias, bias) = packed zero
 };
-
-// diag + (sigma - go) for both halves: base, override when A matches, add when B matches (3 IMADs, no SEL).
-// The match bits of column c sit next to each other in one word (bit 2c: pair A, bit 2c+1: pair B), so that
-// ptxas turns the bit tests of consecutive columns into R2P.
-template <int BIT>
-__device__ __forceinline__ unsigned diag_sigma_x2(unsigned m, unsigned d, const X2Const& k)
-{
-    unsigned dd = (unsigned)diag_plus_sigma_mask<BIT>(m, (int)d, k.one, k.dd_c, k.sd_c);
-    asm("{\n\t.reg .pred p;\n\t.reg .b32 t;\n\tand.b32 t, %1, %2;\n\tsetp.ne.u32 p, t, 0;\n\t@p mad.lo.s32 %0, %3, %4, %0;\n\t}"
-        : "+r"(dd)
-        : "r"(m), "n"(2u << BIT), "r"(k.one), "r"(k.dhi));
-    return dd;
-}
 
 template <int W>
 struct X2State {

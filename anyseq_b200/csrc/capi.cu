@@ -72,6 +72,7 @@ int anyseq_ctx_set_option(anyseq_ctx* ctx, const char* name, int value)
     }
     else if (n == "band_slack" && value >= 1) t.band_slack = value;
     else if (n == "cell_form" && value >= -1 && value <= 2) t.cell_form = value;
+    else if (n == "packed_cells" && value >= -1 && value <= 1) t.packed_cells = value;
     else if (n == "force_generic") t.force_generic = value != 0;
     else if (n == "force_affine") t.force_affine = value != 0;
     else if (n == "local_end_cell") t.local_end_cell = value != 0;
@@ -333,10 +334,22 @@ int anyseq_measure_int_peak(anyseq_ctx* ctx, int kind, double* ops_per_s, float*
     return ctx->eng.measure_int_peak(kind, ops_per_s, sm_mhz_est);
 }
 
+int anyseq_plan_launch_scheme(int sm_count, const anyseq_scoring* sc, int lenq, int lens, int chained, anyseq_launch_plan* out)
+{
+    anyseq::ScoreParams sp;
+    bool affine = false;
+    if (!sc) return ANYSEQ_ERR_BAD_ARG;
+    const int rc = anyseq::make_score_params(*sc, &sp, &affine);
+    if (rc) return rc;
+    anyseq::Engine planner;           // never init()ed: no device, no buffers -- only the planning members are used
+    return planner.plan_launch(sm_count, sc->mode, affine, lenq, lens, chained != 0, sp, out);
+}
+
 int anyseq_plan_launch(int sm_count, int mode, int affine, int lenq, int lens, int chained, anyseq_launch_plan* out)
 {
-    anyseq::Engine planner;           // never init()ed: no device, no buffers -- only the planning members are used
-    return planner.plan_launch(sm_count, mode, affine != 0, lenq, lens, chained != 0, out);
+    // the scheme of the whole-genome benchmark, (2, -1, -2, -1); gap_init = 0 for a linear-gap plan
+    const anyseq_scoring sc = {mode, 2, -1, affine ? -2 : 0, -1};
+    return anyseq_plan_launch_scheme(sm_count, &sc, lenq, lens, chained, out);
 }
 
 int anyseq_device_info(anyseq_ctx* ctx, int* sm_count, int* resident_warps, char* name64)

@@ -173,6 +173,7 @@ using KernelFn = StripKernelFn;
 
 static KernelFn pick_kernel(bool local, bool affine, int K, bool mask, bool track, int form)
 {
+    if (form == 3) return get_strip_kernel_01p(K);
     if (local && track) return affine ? get_strip_kernel_11t(K, mask) : get_strip_kernel_10t(K, mask);
     if (local) return affine ? get_strip_kernel_11(K, mask, form) : get_strip_kernel_10(K, mask, form);
     return affine ? get_strip_kernel_01(K, mask, form) : get_strip_kernel_00(K, mask, form);
@@ -191,6 +192,28 @@ static int pick_form(const Tuning& tune, bool affine, bool mask, int K, long lon
     if (tune.cell_form == 0 || tune.cell_form == 1) return has_coupled ? tune.cell_form : 1;
     if (tune.cell_form == 2) return (has_coupled && K >= 16) ? 2 : 1;
     return (has_coupled && K >= 16 && local && strips_total >= 24LL * sm_count) ? 2 : 1;
+}
+
+// Packed cells (strip_packed.cuh) hold a warp's scores as 16-bit halves around a re-centred offset.  With go = gi + ge,
+// a step right or down changes H by a value in [go, same - go], so every value alive in a warp is within
+// D = max(same - go, -go) per row or column of the others: the warp's live window is 128 rows (64 lanes of two-row
+// tiles) plus 32 rows of drift between two re-centrings, by the strip's 32 * K columns.  It must fit, with the
+// sigma / go constants, into [0x400, 0x7c00] around the centre 0x4000 -- far from 0 and 0xffff, where the IMAD of a
+// packed add would carry into the other half.
+static bool packed_fits(const ScoreParams& sp, int K)
+{
+    if (K != 16 && K != 32) return false;
+    if (sp.gap_open > 0 || sp.gap_extend > 0 || sp.gap_open > sp.gap_extend || sp.same < sp.diff) return false;
+    const long long D = std::max<long long>((long long)sp.same - sp.gap_open, -(long long)sp.gap_open);
+    const long long constants = 4LL * (std::llabs(sp.same) + std::llabs(sp.diff) + std::llabs(sp.gap_open));
+    return D * (128 + 32 + 32LL * K) + constants <= 0x3c00;
+}
+
+// Packed cells for a global / semiglobal Gotoh score launch (MASK kernels, K = 16 or 32) whose window fits; the
+// option packed_cells = 0 keeps the 32-bit decoupled cells.
+static bool use_packed(const Tuning& tune, const ScoreParams& sp, bool local, bool affine, bool mask, bool track, int K)
+{
+    return tune.packed_cells != 0 && !local && affine && mask && !track && packed_fits(sp, K);
 }
 
 // rows per lane and step of the kernel variant (strip_kernel.cuh: StripRows)
@@ -223,23 +246,24 @@ static int default_blocks_per_sm(int K, bool mask, bool track, int occupancy_max
     return nb;
 }
 
-// dynamic shared memory of the MASK kernels: [warps][ncodes][32 lanes][W words] spread column masks
-static size_t mask_smem_bytes(bool mask, bool track, int ncodes, int K, int warps)
+// dynamic shared memory of the MASK kernels: [warps][ncodes][32 lanes][W words] spread column masks (packed cells:
+// one set per half of the strip)
+static size_t mask_smem_bytes(bool mask, bool track, int ncodes, int K, int warps, int form)
 {
     if (!mask) return 0;
-    const int words = std::max(1, rows_per_step(K, mask, track) * K / 32);
+    const int words = std::max(1, rows_per_step(K, mask, track) * K / 32) * (form == 3 ? 2 : 1);
     return sizeof(unsigned) * 32 * (size_t)ncodes * warps * words;
 }
 
 // Launch shape of a strip kernel: the end-cell tracking kernels run `nb` CTAs of 4 warps per SM, all others ONE CTA of
 // 4 * nb warps per SM (strip_kernel.cuh: the warps of a scheduler take adjacent strips).  Returns the largest nb <= want
 // that fits, 0 if none does.
-static int fit_blocks_per_sm(KernelFn fn, bool track, bool mask, int ncodes, int K, int want)
+static int fit_blocks_per_sm(KernelFn fn, bool track, bool mask, int ncodes, int K, int want, int form)
 {
     for (int nb = want; nb >= 1; --nb) {
         int got = 0;
         const int warps = track ? kWarpsPerBlock : kWarpsPerBlock * nb;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, fn, warps * kWarp, mask_smem_bytes(mask, track, ncodes, K, warps)) != cudaSuccess)
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&got, fn, warps * kWarp, mask_smem_bytes(mask, track, ncodes, K, warps, form)) != cudaSuccess)
             return 0;
         if (track ? got >= nb : got >= 1) return nb;
     }
@@ -342,6 +366,7 @@ int Engine::init(int dev)
     if ((env = std::getenv("ANYSEQ_ALIGN_SCORE"))) tune.align_with_score = std::atoi(env) != 0;
     if ((env = std::getenv("ANYSEQ_FORCE_GENERIC"))) tune.force_generic = std::atoi(env) != 0;
     if ((env = std::getenv("ANYSEQ_CELL_FORM"))) tune.cell_form = std::atoi(env);
+    if ((env = std::getenv("ANYSEQ_PACKED_CELLS"))) tune.packed_cells = std::atoi(env);
     if ((env = std::getenv("ANYSEQ_SMALL_MODEL"))) tune.small_model = std::atoi(env) != 0;
     if ((env = std::getenv("ANYSEQ_BATCH_PACKED"))) tune.batch_packed = std::atoi(env) != 0;
     if ((env = std::getenv("ANYSEQ_BATCH_QUAD"))) tune.batch_quad = std::atoi(env) != 0;
@@ -386,7 +411,7 @@ int Engine::resident_warps(int K, bool local, bool affine, long long nstrips)
     const bool track = track_ && local;
     int want = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, use_mask_, track, track ? 6 : 3, nstrips, sm_count, form);
     if (!track) want = std::min(want, kMaxStripWarps / kWarpsPerBlock);
-    return fit_blocks_per_sm(fn, track, use_mask_, ncodes_, K, want) * kWarpsPerBlock * sm_count;
+    return fit_blocks_per_sm(fn, track, use_mask_, ncodes_, K, want, form) * kWarpsPerBlock * sm_count;
 }
 
 // Decide between the MASK and the generic kernels for a (query, subject) pair
@@ -532,7 +557,8 @@ int Engine::balance_warps(int nb, int max_h, long long strips_total, int K, bool
 // this engine's `tune` says otherwise) on a GPU with `sms` SMs -- host logic only, no CUDA call: what the CPU tests and
 // tools/plan.py look at.  The occupancy query of the real path (fit_blocks_per_sm) is taken as granted; the shipped
 // kernels fit 12 warps per SM.
-int Engine::plan_launch(int sms, int mode, bool affine, int m, int n, bool chained, anyseq_launch_plan* out)
+int Engine::plan_launch(int sms, int mode, bool affine, int m, int n, bool chained, const ScoreParams& sp,
+                        anyseq_launch_plan* out)
 {
     if (sms < 1 || m < 1 || n < 1 || mode < 0 || mode > 2 || !out) { set_last_error("bad plan request"); return ANYSEQ_ERR_BAD_ARG; }
     sm_count = sms;
@@ -561,12 +587,13 @@ int Engine::plan_launch(int sms, int mode, bool affine, int m, int n, bool chain
     out->grid = grid;
     out->warps_per_cta = wpb;
     out->first_items = first;
+    out->packed_cells = (!chained && use_packed(tune, sp, local, affine, true, false, K)) ? 1 : 0;
     return ANYSEQ_OK;
 }
 
 // Launch init + strip kernels for a job list that is already in host memory.
 int Engine::run_jobs(std::vector<Job>& jobs, const ScoreParams& sp, bool local, bool affine, int K,
-                     int* launches)
+                     int* launches, bool packed_ok)
 {
     const int njobs = (int)jobs.size();
     long long strips_total = 0;
@@ -578,15 +605,16 @@ int Engine::run_jobs(std::vector<Job>& jobs, const ScoreParams& sp, bool local, 
     }
     if (strips_total > 0x7fffffff) { set_last_error("too many strips in one launch"); return ANYSEQ_ERR_UNSUPPORTED; }
 
-    const int form = pick_form(tune, affine, use_mask_, K, strips_total, sm_count, local);
-    KernelFn fn = pick_kernel(local, affine, K, use_mask_, track_ && local, form);
-    if (!fn) { set_last_error("unsupported columns-per-lane"); return ANYSEQ_ERR_BAD_ARG; }
     const bool track = track_ && local;
     bool chained = false;
     for (const Job& j : jobs) chained = chained || j.in != nullptr || j.out != nullptr;
+    const bool packed = packed_ok && !chained && use_packed(tune, sp, local, affine, use_mask_, track, K);
+    const int form = packed ? 3 : pick_form(tune, affine, use_mask_, K, strips_total, sm_count, local);
+    KernelFn fn = pick_kernel(local, affine, K, use_mask_, track_ && local, form);
+    if (!fn) { set_last_error("unsupported columns-per-lane"); return ANYSEQ_ERR_BAD_ARG; }
     int want = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, use_mask_, track, track ? 6 : 3, strips_total, sm_count, form);
     if (!track) want = balance_warps(std::min(want, kMaxStripWarps / kWarpsPerBlock), max_h, strips_total, K, chained);
-    const int nb = fit_blocks_per_sm(fn, track, use_mask_, ncodes_, K, want);
+    const int nb = fit_blocks_per_sm(fn, track, use_mask_, ncodes_, K, want, form);
     if (nb < 1) { set_last_error("strip kernel does not fit on an SM"); return ANYSEQ_ERR_UNSUPPORTED; }
     const int resident = nb * kWarpsPerBlock * sm_count;
 
@@ -662,7 +690,7 @@ int Engine::run_jobs(std::vector<Job>& jobs, const ScoreParams& sp, bool local, 
     ANYSEQ_CUDA_CHECK(cudaEventRecord(g_ev_k0, stream_));
 #endif
     ANYSEQ_CUDA_CHECK(cudaLaunchCooperativeKernel((const void*)fn, dim3(grid), dim3(wpb_used * kWarp), args,
-                                                  mask_smem_bytes(use_mask_, track, ncodes_, K, wpb_used), stream_));
+                                                  mask_smem_bytes(use_mask_, track, ncodes_, K, wpb_used, form), stream_));
 #ifdef ANYSEQ_PROFILE
     ANYSEQ_CUDA_CHECK(cudaEventRecord(g_ev_k1, stream_));
     std::fprintf(stderr, "[anyseq profile] launch: grid=%d warps/CTA=%d items=%lld bands=%d form=%d\n", grid, wpb_used, total, nbands, form);
@@ -794,7 +822,8 @@ int Engine::score_strip_device(const anyseq_scoring& sc, const uint8_t* d_q, int
     int launches = 0;
     init_col0_ = col_begin;
     launches += 3;   // alphabet analysis
-    rc = run_jobs(jobs, sp, local, affine, K, &launches);
+    // packed cells for whole single-GPU score problems (not for the edge columns of a full-matrix traceback)
+    rc = run_jobs(jobs, sp, local, affine, K, &launches, whole && !want_edges_);
     init_col0_ = 0;
     if (rc) return rc;
     finish_score_kernel<<<1, 1024, 0, stream_>>>(jobs_.as<Job>(), sc.mode, col_begin, n_total,

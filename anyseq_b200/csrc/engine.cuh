@@ -42,6 +42,7 @@ struct Tuning {
     int blocks_per_sm = 0;   // 0 = occupancy maximum
     int watchdog_ms = 20000;
     int cell_form = -1;      // -1 = per launch (engine.cu: pick_form), 0 = coupled, 1 = decoupled cells
+    int packed_cells = -1;   // -1 / 1 = packed cells where the score window fits (engine.cu: packed_fits), 0 = never
     int band_slack = 2;      // band height = band_slack * lag * (resident warps) when the strips outnumber the warps
     bool force_generic = false;     // never use the MASK kernels (testing)
     bool force_affine = false;      // score path: run the Gotoh kernels even for gap_init == 0 (testing: must equal the linear kernels)
@@ -129,7 +130,8 @@ public:
                                  anyseq_result* out);
     int measure_int_peak(int kind, double* ops_per_s, float* sm_mhz);
     // launch planning without a device (engine.cu); usable on an Engine that was never init()ed
-    int plan_launch(int sms, int mode, bool affine, int m, int n, bool chained, anyseq_launch_plan* out);
+    int plan_launch(int sms, int mode, bool affine, int m, int n, bool chained, const ScoreParams& sp,
+                    anyseq_launch_plan* out);
 
     int inbox_create(int rows, Inbox** out, void* handle64);
     int inbox_open(const void* handle64, int rows, Inbox** out);
@@ -148,7 +150,8 @@ public:
     void drop_host_batch_stream();       // batch_stream.cu: the cached pipeline of score_batch_host
 
 private:
-    int run_jobs(std::vector<Job>& jobs, const ScoreParams& sp, bool local, bool affine, int K, int* launches);
+    int run_jobs(std::vector<Job>& jobs, const ScoreParams& sp, bool local, bool affine, int K, int* launches,
+                 bool packed_ok = false);
     int pick_K(int n, bool chained = false, int m = 0, bool affine = false) const;
     int pick_K_levels(int n_total) const;
     int analyse_alphabet(const uint8_t* d_q, long long m, const uint8_t* d_s, long long n);

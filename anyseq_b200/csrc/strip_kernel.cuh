@@ -45,7 +45,9 @@ namespace anyseq {
 //                   win the maximum that forms E(i,j) (E+go <= E+ge).  A lone warp saturates its scheduler's ALU pipe, so
 //                   half as many (twice as fast) warps are needed -- which is what the strip-to-strip chain, narrow
 //                   problems and multi-GPU slices are sensitive to.
-// Both forms are built (template parameter FORM of strip_kernel); engine.cu picks per launch: the coupled form where
+//   3  "packed":    the decoupled cell on 16-bit halves, two cells per DPX instruction (strip_packed.cuh; global and
+//                   semiglobal Gotoh with column masks, when the scheme's score window fits 16 bits).
+// The forms are built as template parameter FORM of strip_kernel; engine.cu picks per launch: the coupled form where
 // three warps per scheduler can be fed (Gotoh, strips >> warps: 3.71 vs 3.52 TCUPS on the 4.6 Mbp pair), the decoupled
 // form everywhere else (linear gaps, single-band launches, small problems, multi-GPU slices).
 
@@ -481,7 +483,8 @@ struct CellR {
 struct alignas(16) WarpSmem {
     int2 in[32];        // left border rows of the current batch (X form, E)
     int2 out[64];       // right edge rows waiting to be published (ring of two batches)
-    uint8_t q[256];     // query symbols (MASK: codes) of the last 64*R rows (ring)
+    uint8_t q[256];     // query symbols (MASK: codes) of the last 64*R rows (ring; packed cells: the last 256 rows)
+    int boff[8];        // packed cells: the warp's score offset of each of the last 8 batches (strip_packed.cuh)
 };
 
 __device__ __forceinline__ int4 ld_record(const int4* p)
@@ -900,6 +903,12 @@ __device__ __forceinline__ bool process_item(const Job& J, const int band, const
     return true;
 }
 
+}  // namespace anyseq
+
+#include "strip_packed.cuh"
+
+namespace anyseq {
+
 // rows per lane and step of each kernel variant
 #ifndef ANYSEQ_ROWS_K32
 #define ANYSEQ_ROWS_K32 2
@@ -950,7 +959,9 @@ strip_kernel(const KernelArgs a)
         }
         __syncthreads();
     }
-    unsigned* s_mask = s_dyn + warp * a.ncodes * 32 * TileWords<R, K>::value;
+    static_assert(FORM != 3 || (!LOCAL && AFFINE && MASK && !TRACK && R == 2), "packed cells: global / semiglobal Gotoh two-row MASK tiles");
+    // packed cells keep one mask per half of the strip
+    unsigned* s_mask = s_dyn + warp * a.ncodes * 32 * TileWords<R, K>::value * (FORM == 3 ? 2 : 1);
     // the query ring is read one row ahead (mask prefetch): never let an
     // uninitialised byte be used as a code
     for (int x = lane; x < 256; x += 32) s_warp[warp].q[x] = 0;
@@ -991,6 +1002,9 @@ strip_kernel(const KernelArgs a)
         bool ok = true;
         if ((long long)band * J.band_h >= J.h) {
             // a band past the end of a short job: nothing to relax
+        } else if constexpr (FORM == 3) {
+            if (partial) ok = process_item_packed<K, 1>(J, band, strip, a, s_warp[warp], s_mask, s_lut, lane);
+            else ok = process_item_packed<K, 0>(J, band, strip, a, s_warp[warp], s_mask, s_lut, lane);
         } else if (partial) {
             ok = process_item<LOCAL, AFFINE, K, 1, MASK, R, TRACK, FORM>(J, band, strip, a, s_warp[warp], s_mask, s_lut, lane);
         } else {
@@ -1012,5 +1026,6 @@ StripKernelFn get_strip_kernel_10(int K, bool mask, int form);
 StripKernelFn get_strip_kernel_11(int K, bool mask, int form);
 StripKernelFn get_strip_kernel_10t(int K, bool mask);   // local + end-cell tracking
 StripKernelFn get_strip_kernel_11t(int K, bool mask);
+StripKernelFn get_strip_kernel_01p(int K);              // global / semiglobal Gotoh, packed cells (strip_packed.cuh)
 
 }  // namespace anyseq

@@ -343,8 +343,12 @@ typedef struct anyseq_launch_plan {
     int32_t grid;                 /* CTAs (one per SM at most) */
     int32_t warps_per_cta;
     int64_t first_items;          /* (band, strip) items assigned statically; the rest is claimed from a counter */
+    int32_t packed_cells;         /* 1: the decoupled Gotoh cells run as 16-bit pairs, two per DPX instruction (DESIGN.md 3.1) */
 } anyseq_launch_plan;
+/* anyseq_plan_launch answers for the scheme (same, diff, gap_init, gap_extend) = (2, -1, -2, -1) (gap_init = 0 when
+ * affine == 0); anyseq_plan_launch_scheme for any scheme (packed_cells depends on it). */
 int anyseq_plan_launch(int sm_count, int mode, int affine, int lenq, int lens, int chained, anyseq_launch_plan* out);
+int anyseq_plan_launch_scheme(int sm_count, const anyseq_scoring* sc, int lenq, int lens, int chained, anyseq_launch_plan* out);
 
 #ifdef __cplusplus
 }
