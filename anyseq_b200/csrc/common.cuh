@@ -67,8 +67,6 @@ struct Job {
     int4* out;
     int in_tag;
     int out_tag;
-    int edge_e;              // 1: a ragged last strip must also keep E of the matrix's last column (Gotoh traceback joins,
-                             // mirrors to a next rank); 0: H only (cheaper ragged strips)
     // initialisation of the borders (init kernel)
     int init_global;         // 1: gap multiples (global), 0: zeros
     int top_open;            // global: H(-1, j) = top_open + j * gap_extend (cost of the first gap symbol on

@@ -816,7 +816,6 @@ int Engine::score_strip_device(const anyseq_scoring& sc, const uint8_t* d_q, int
     // the tag of a run is agreed without communication: both ends count their uses of the inbox
     if (inbox) { J.in = inbox->records; J.in_tag = 0x40000000 + (++inbox->uses_in & 0xffffff); }
     if (next_inbox) { J.out = next_inbox->records; J.out_tag = 0x40000000 + (++next_inbox->uses_out & 0xffffff); }
-    J.edge_e = (next_inbox != nullptr || want_edges_) ? 1 : 0;     // who reads E of a ragged last strip's edge column
 
     std::vector<Job> jobs(1, J);
     int launches = 0;
@@ -982,7 +981,6 @@ int Engine::score_strip_device_multi(const anyseq_scoring& sc, int npairs, const
         Inbox* nx = next_inbox ? next_inbox[p] : nullptr;
         if (in) { J.in = in->records; J.in_tag = 0x40000000 + (++in->uses_in & 0xffffff); }
         if (nx) { J.out = nx->records; J.out_tag = 0x40000000 + (++nx->uses_out & 0xffffff); }
-        J.edge_e = nx ? 1 : 0;
     }
     int launches = 2 * npairs + 1;   // alphabet analysis
     init_col0_ = col_begin;

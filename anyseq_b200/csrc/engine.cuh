@@ -108,8 +108,6 @@ public:
                                  Inbox* const* inbox, Inbox* const* next_inbox, anyseq_strip_partial* out);
     int align_host(const anyseq_scoring& sc, const char* q, int m, const char* s, int n,
                    char* alq, char* als, anyseq_result* out);
-    int align_host_affine(const anyseq_scoring& sc, const char* q, int m, const char* s, int n,
-                          char* alq, char* als, anyseq_result* out);
     // this rank's share of a traceback spread over `shard.world` GPUs (traceback.cu); alq/als are full-size buffers of
     // which only [shard.out_lo, shard.out_hi) is meaningful afterwards
     int align_host_sharded(const anyseq_scoring& sc, const char* q, int m, const char* s, int n,
