@@ -21,14 +21,13 @@
 
 namespace anyseq {
 
-// stats[0] = max over pairs of max(lenq, lens), stats[1] = max over pairs of min(lenq, lens)
-__global__ void batch_stats_kernel(const long long* __restrict__ qoff, const long long* __restrict__ soff,
-                                   long long npairs, int* __restrict__ stats)
+// stats[0] = max over pairs of max(lenq, lens), stats[1] = max over pairs of min(lenq, lens), clamped to 2^31 - 1
+__global__ void batch_stats_kernel(const BatchArgs a, int* __restrict__ stats)
 {
     int mx = 0, mn = 0;
-    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < npairs; p += (long long)gridDim.x * blockDim.x) {
-        const long long a = qoff[p + 1] - qoff[p], b = soff[p + 1] - soff[p];
-        const long long hi = a > b ? a : b, lo = a > b ? b : a;
+    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < a.npairs; p += (long long)gridDim.x * blockDim.x) {
+        const long long lq = batch_q_len(a, p), ls = batch_s_len(a, p);
+        const long long hi = lq > ls ? lq : ls, lo = lq > ls ? ls : lq;
         mx = max(mx, (int)min(hi, (long long)0x7fffffff));
         mn = max(mn, (int)min(lo, (long long)0x7fffffff));
     }
@@ -37,17 +36,6 @@ __global__ void batch_stats_kernel(const long long* __restrict__ qoff, const lon
         mn = max(mn, __shfl_xor_sync(0xffffffffu, mn, o));
     }
     if ((threadIdx.x & 31) == 0) { atomicMax(&stats[0], mx); atomicMax(&stats[1], mn); }
-}
-
-// value of X[idx] for a run-time idx (one lane needs it; jump table, not K selects)
-template <int K>
-__device__ __forceinline__ int pick_column(const int (&X)[K], int idx)
-{
-    int v = X[0];
-#pragma unroll
-    for (int c = 1; c < K; ++c)
-        if (c == idx) v = X[c];
-    return v;
 }
 
 template <int MODE, bool AFFINE, int K, bool MASK>
@@ -89,9 +77,7 @@ __global__ void __launch_bounds__(kThreads, (K >= 32 ? 4 : (K >= 16 ? 5 : 6))) b
         const int lq = batch_q_len(a, pair), ls = batch_s_len(a, pair);
         int score;
         if (lq == 0 || ls == 0) {
-            // quirk Q12 (see engine.cu: empty_result)
-            const int L = max(lq, ls);
-            score = GLOB ? (L > 0 ? a.gap_init + L * a.sp.gap_extend : 0) : (MODE == kSemiglobal ? 0 : kScoreMin);
+            score = empty_pair_score<MODE>(a, lq, ls);
         } else {
             const bool q_is_cols = a.cols_longer ? (lq >= ls) : (lq < ls);
             const uint8_t* cols = q_is_cols ? a.q + q0 : a.s + s0;
@@ -166,7 +152,7 @@ __global__ void __launch_bounds__(kThreads, (K >= 32 ? 4 : (K >= 16 ? 5 : 6))) b
                         hr = st.xleft;
                         er = st.e;
                         if constexpr (MODE == kSemiglobal) {
-                            if (lane == outlane) colbest = max(colbest, pick_column<K>(X, outc));
+                            if (lane == outlane) colbest = max(colbest, pick_column(X, outc));
                         }
                     }
                     if constexpr (MASK) st.tm[0] = mask_next;
@@ -174,7 +160,7 @@ __global__ void __launch_bounds__(kThreads, (K >= 32 ? 4 : (K >= 16 ? 5 : 6))) b
             }
             // result extraction: src/scoring.impala:29-137 (values only)
             if constexpr (GLOB) {
-                score = __shfl_sync(kFull, pick_column<K>(X, outc), outlane) - go;
+                score = __shfl_sync(kFull, pick_column(X, outc), outlane) - go;
             } else if constexpr (MODE == kSemiglobal) {
                 int best = colbest;
 #pragma unroll
@@ -260,19 +246,21 @@ int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool a
         const long long small = std::max<long long>({std::llabs(sc.same), std::llabs(sc.diff), std::llabs(go), std::llabs(sc.gap_extend)});
         if (b + hmax + 2 * small < 32000 && small < 2000) { packed = true; bias = (int)b; }
     }
-    // four pairs per warp (half-warps, batch_x2.cu: batch_x4_kernel) when the column sequences fit 16 lanes x 32 columns
+    // four pairs per warp (groups of 16 lanes x 32 columns) when the column sequences fit a half-warp
     const bool quad = packed && tune.batch_quad && ncols <= 512;
-    BatchKernelFn fn = quad ? pick_batch_x4_kernel(sc.mode, affine)
-                            : (packed ? pick_batch_x2_kernel(sc.mode, affine, K) : pick_batch_kernel(sc.mode, affine, K, use_mask_));
+    const int lanes = quad ? 16 : 32;     // lanes per group; a packed group relaxes two pairs
+    if (quad) K = 32;
+    BatchKernelFn fn = packed ? pick_batch_x2_kernel(sc.mode, affine, K, lanes) : pick_batch_kernel(sc.mode, affine, K, use_mask_);
     if (!fn) { set_last_error("no batch kernel for this configuration"); return ANYSEQ_ERR_UNSUPPORTED; }
-    // packed: two mask sets, match bits spread to every other bit (2 K bits per lane and row); quad: per half-warp, K = 32
-    const size_t dyn = !use_mask_ ? 0
-                       : quad ? sizeof(unsigned) * 16 * (size_t)ncodes_ * kWarpsPerBlock * 2 * 2 * 2
-                              : sizeof(unsigned) * 32 * (size_t)ncodes_ * kWarpsPerBlock * (packed ? 2 * ((2 * K + 31) / 32) : 1);
+    // one column-mask set per pair of a warp, W words per lane, code and row; packed kernels spread the match bits to
+    // every other bit (2 K bits per lane and row)
+    const int W = packed ? (2 * K + 31) / 32 : 1;
+    const int pairs_per_warp = packed ? 2 * (32 / lanes) : 1;
+    const size_t dyn = use_mask_ ? sizeof(unsigned) * lanes * W * (size_t)ncodes_ * pairs_per_warp * kWarpsPerBlock : 0;
     int nb = 0;
     ANYSEQ_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, kThreads, dyn));
     if (nb < 1) { set_last_error("batch kernel does not fit on an SM"); return ANYSEQ_ERR_UNSUPPORTED; }
-    const long long units = quad ? (npairs + 3) / 4 : (packed ? (npairs + 1) / 2 : npairs);      // work items claimed by the warps
+    const long long units = (npairs + pairs_per_warp - 1) / pairs_per_warp;      // work items claimed by the warps
     const int grid = (int)std::min<long long>((long long)nb * sm_count, (units + kWarpsPerBlock - 1) / kWarpsPerBlock);
     ba.sp = sp;
     ba.gap_init = sc.gap_init;
@@ -290,6 +278,41 @@ int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool a
     return ANYSEQ_OK;
 }
 
+int batch_prologue(const anyseq_scoring& sc, int64_t npairs, ScoreParams* sp, bool* affine, anyseq_result* out)
+{
+    const int rc = make_score_params(sc, sp, affine);
+    if (rc) return rc;
+    if (out) { std::memset(out, 0, sizeof(*out)); out->end_i = out->end_j = -1; }
+    if (npairs > 0 && sc.mode == ANYSEQ_LOCAL && sc.diff > 0) {
+        set_last_error("batch local alignment needs diff <= 0 (padded columns must not outscore real ones)");
+        return ANYSEQ_ERR_UNSUPPORTED;
+    }
+    return ANYSEQ_OK;
+}
+
+int Engine::batch_len_stats(const BatchArgs& ba, int* max_long, int* max_short)
+{
+    int* d_stats = misc_.as<int>() + kMiscOut;
+    ANYSEQ_CUDA_CHECK(cudaMemsetAsync(d_stats, 0, sizeof(int) * 2, stream_));
+    batch_stats_kernel<<<(int)std::min<long long>(sm_count * 8, (ba.npairs + 255) / 256), 256, 0, stream_>>>(ba, d_stats);
+    ANYSEQ_CUDA_CHECK(cudaGetLastError());
+    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(h_misc_ + kMiscOut, d_stats, sizeof(int) * 2, cudaMemcpyDeviceToHost, stream_));
+    ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    *max_long = h_misc_[kMiscOut];
+    *max_short = h_misc_[kMiscOut + 1];
+    return ANYSEQ_OK;
+}
+
+int Engine::batch_epilogue(int launches, anyseq_result* out)
+{
+    ANYSEQ_CUDA_CHECK(cudaEventRecord(ev1_, stream_));
+    ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    float ms = 0.f;
+    ANYSEQ_CUDA_CHECK(cudaEventElapsedTime(&ms, ev0_, ev1_));
+    if (out) { out->kernel_ms = ms; out->kernel_launches = launches; }
+    return ANYSEQ_OK;
+}
+
 int Engine::score_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, const int64_t* d_qoff,
                                const uint8_t* d_s, const int64_t* d_soff, int64_t npairs, int32_t* d_scores,
                                anyseq_result* out)
@@ -298,29 +321,9 @@ int Engine::score_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, con
     ANYSEQ_CUDA_CHECK(cudaSetDevice(device));
     ScoreParams sp;
     bool affine;
-    int rc = make_score_params(sc, &sp, &affine);
-    if (rc) return rc;
-    if (out) { std::memset(out, 0, sizeof(*out)); out->end_i = out->end_j = -1; }
-    if (npairs == 0) return ANYSEQ_OK;
-    if (sc.mode == ANYSEQ_LOCAL && sc.diff > 0) {
-        set_last_error("batch local alignment needs diff <= 0 (padded columns must not outscore real ones)");
-        return ANYSEQ_ERR_UNSUPPORTED;
-    }
+    int rc = batch_prologue(sc, npairs, &sp, &affine, out);
+    if (rc || npairs == 0) return rc;
     ANYSEQ_CUDA_CHECK(cudaEventRecord(ev0_, stream_));
-    // totals (for the alphabet scan) and length statistics
-    long long tot[2] = {0, 0};
-    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(&tot[0], d_qoff + npairs, sizeof(long long), cudaMemcpyDeviceToHost, stream_));
-    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(&tot[1], d_soff + npairs, sizeof(long long), cudaMemcpyDeviceToHost, stream_));
-    int* d_stats = misc_.as<int>() + kMiscOut;
-    ANYSEQ_CUDA_CHECK(cudaMemsetAsync(d_stats, 0, sizeof(int) * 2, stream_));
-    batch_stats_kernel<<<(int)std::min<long long>(sm_count * 8, (npairs + 255) / 256), 256, 0, stream_>>>(
-        reinterpret_cast<const long long*>(d_qoff), reinterpret_cast<const long long*>(d_soff), npairs, d_stats);
-    ANYSEQ_CUDA_CHECK(cudaGetLastError());
-    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(h_misc_ + kMiscOut, d_stats, sizeof(int) * 2, cudaMemcpyDeviceToHost, stream_));
-    ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
-    const int max_long = h_misc_[kMiscOut], max_short = h_misc_[kMiscOut + 1];
-    rc = analyse_alphabet(d_q, tot[0], d_s, tot[1]);
-    if (rc) return rc;
     BatchArgs ba;
     std::memset(&ba, 0, sizeof(ba));
     ba.q = d_q;
@@ -329,14 +332,15 @@ int Engine::score_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, con
     ba.soff = reinterpret_cast<const long long*>(d_soff);
     ba.npairs = npairs;
     ba.scores = d_scores;
-    rc = launch_batch(sc, sp, affine, ba, max_long, max_short, stream_);
-    if (rc) return rc;
-    ANYSEQ_CUDA_CHECK(cudaEventRecord(ev1_, stream_));
-    ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
-    float ms = 0.f;
-    ANYSEQ_CUDA_CHECK(cudaEventElapsedTime(&ms, ev0_, ev1_));
-    if (out) { out->kernel_ms = ms; out->kernel_launches = 5; }
-    return ANYSEQ_OK;
+    // totals (for the alphabet scan) and length statistics
+    long long tot[2] = {0, 0};
+    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(&tot[0], d_qoff + npairs, sizeof(long long), cudaMemcpyDeviceToHost, stream_));
+    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(&tot[1], d_soff + npairs, sizeof(long long), cudaMemcpyDeviceToHost, stream_));
+    int max_long, max_short;
+    if ((rc = batch_len_stats(ba, &max_long, &max_short))) return rc;
+    if ((rc = analyse_alphabet(d_q, tot[0], d_s, tot[1]))) return rc;
+    if ((rc = launch_batch(sc, sp, affine, ba, max_long, max_short, stream_))) return rc;
+    return batch_epilogue(5, out);
 }
 
 }  // namespace anyseq

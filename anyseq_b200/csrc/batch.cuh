@@ -1,4 +1,4 @@
-// batch.cuh -- argument block shared by the batch kernels (batch.cu, batch_x2.cu)
+// batch.cuh -- argument block and device helpers shared by the batch kernels (batch.cu, batch_x2.cu)
 #pragma once
 #include "common.cuh"
 
@@ -33,13 +33,14 @@ struct BatchArgs {
 // where pair p's sequences start (symbol offset, or byte offset for 2-bit input) and how many symbols they have
 __device__ __forceinline__ long long batch_q_start(const BatchArgs& a, long long p) { return a.qoff ? a.qoff[p] : p * a.qstride; }
 __device__ __forceinline__ long long batch_s_start(const BatchArgs& a, long long p) { return a.soff ? a.soff[p] : p * a.sstride; }
-__device__ __forceinline__ int batch_q_len(const BatchArgs& a, long long p)
+// 64-bit so that the length statistics see a pair of 2^31 or more symbols as too long; the kernels take it as int
+__device__ __forceinline__ long long batch_q_len(const BatchArgs& a, long long p)
 {
-    return a.packed2 ? (a.qlen ? a.qlen[p] : a.qlen_u) : (int)(a.qoff[p + 1] - a.qoff[p]);
+    return a.packed2 ? (a.qlen ? a.qlen[p] : a.qlen_u) : a.qoff[p + 1] - a.qoff[p];
 }
-__device__ __forceinline__ int batch_s_len(const BatchArgs& a, long long p)
+__device__ __forceinline__ long long batch_s_len(const BatchArgs& a, long long p)
 {
-    return a.packed2 ? (a.slen ? a.slen[p] : a.slen_u) : (int)(a.soff[p + 1] - a.soff[p]);
+    return a.packed2 ? (a.slen ? a.slen[p] : a.slen_u) : a.soff[p + 1] - a.soff[p];
 }
 // alphabet code of symbol idx of a sequence: byte -> code table, or the 2-bit value + 1 (code 0 matches nothing)
 __device__ __forceinline__ int batch_code(const uint8_t* __restrict__ base, int idx, int packed2, const uint8_t* lut)
@@ -48,10 +49,28 @@ __device__ __forceinline__ int batch_code(const uint8_t* __restrict__ base, int 
     return (int)lut[base[idx]];
 }
 
+// score of a pair with an empty sequence, following the reference's storage (quirk Q12, see engine.cu: empty_result)
+template <int MODE>
+__device__ __forceinline__ int empty_pair_score(const BatchArgs& a, int lq, int ls)
+{
+    const int L = max(lq, ls);
+    return MODE == kGlobal ? (L > 0 ? a.gap_init + L * a.sp.gap_extend : 0) : (MODE == kSemiglobal ? 0 : kScoreMin);
+}
+
+// value of X[idx] for a run-time idx (one lane needs it; jump table, not K selects)
+template <typename T, int K>
+__device__ __forceinline__ T pick_column(const T (&X)[K], int idx)
+{
+    T v = X[0];
+#pragma unroll
+    for (int c = 1; c < K; ++c)
+        if (c == idx) v = X[c];
+    return v;
+}
+
 using BatchKernelFn = void (*)(const BatchArgs);
-// packed 16-bit kernels (batch_x2.cu): two pairs of equal shape per warp; nullptr if K is not instantiated
-BatchKernelFn pick_batch_x2_kernel(int mode, bool affine, int K);
-// four pairs per warp (16 lanes x 32 columns per pair of pairs): column sequences of at most 512 symbols
-BatchKernelFn pick_batch_x4_kernel(int mode, bool affine);
+// packed 16-bit kernels (batch_x2.cu): two pairs per group of `lanes` lanes (32: K = 4, 8, 16, 32; 16: K = 32, four
+// pairs per warp); nullptr for other combinations
+BatchKernelFn pick_batch_x2_kernel(int mode, bool affine, int K, int lanes);
 
 }  // namespace anyseq

@@ -17,24 +17,8 @@
 
 namespace anyseq {
 
-// stats[0] = max over pairs of max(lenq, lens), stats[1] = max over pairs of min(lenq, lens)
-__global__ void batch_len_stats_kernel(const int* __restrict__ qlen, const int* __restrict__ slen, int qlen_u, int slen_u,
-                                       long long npairs, int* __restrict__ stats)
-{
-    int mx = 0, mn = 0;
-    for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < npairs; p += (long long)gridDim.x * blockDim.x) {
-        const int a = qlen ? qlen[p] : qlen_u, b = slen ? slen[p] : slen_u;
-        mx = max(mx, max(a, b));
-        mn = max(mn, min(a, b));
-    }
-    for (int o = 16; o > 0; o >>= 1) {
-        mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-        mn = max(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-    }
-    if ((threadIdx.x & 31) == 0) { atomicMax(&stats[0], mx); atomicMax(&stats[1], mn); }
-}
-
-static int check_packed_batch(const anyseq_packed_batch& b)
+// the caller's description of a 2-bit batch and its score array
+static int check_packed_batch(const anyseq_packed_batch& b, const int32_t* scores)
 {
     if (b.npairs < 0 || (b.npairs > 0 && (!b.q2 || !b.s2))) { set_last_error("packed batch: null sequence arrays"); return ANYSEQ_ERR_BAD_ARG; }
     if ((!b.q_len && b.q_len_uniform < 0) || (!b.s_len && b.s_len_uniform < 0)) { set_last_error("packed batch: negative length"); return ANYSEQ_ERR_BAD_ARG; }
@@ -43,7 +27,15 @@ static int check_packed_batch(const anyseq_packed_batch& b)
         set_last_error("packed batch: stride shorter than a packed sequence");
         return ANYSEQ_ERR_BAD_ARG;
     }
+    if (b.npairs > 0 && !scores) { set_last_error("packed batch: null score array"); return ANYSEQ_ERR_BAD_ARG; }
     return ANYSEQ_OK;
+}
+
+int Engine::use_2bit_alphabet()
+{
+    use_mask_ = true;
+    ncodes_ = 5;
+    return lut_.ensure(512 + 64 + 16) ? ANYSEQ_ERR_NO_DEVICE : ANYSEQ_OK;
 }
 
 static void fill_args(BatchArgs& ba, const anyseq_packed_batch& b, int32_t* d_scores)
@@ -71,47 +63,22 @@ int Engine::score_batch_packed2_device(const anyseq_scoring& sc, const anyseq_pa
     ANYSEQ_CUDA_CHECK(cudaSetDevice(device));
     ScoreParams sp;
     bool affine;
-    int rc = make_score_params(sc, &sp, &affine);
+    int rc = check_packed_batch(b, d_scores);
     if (rc) return rc;
-    if ((rc = check_packed_batch(b))) return rc;
-    if (out) { std::memset(out, 0, sizeof(*out)); out->end_i = out->end_j = -1; }
-    if (b.npairs == 0) return ANYSEQ_OK;
-    if (!d_scores) { set_last_error("packed batch: null score array"); return ANYSEQ_ERR_BAD_ARG; }
-    if (sc.mode == ANYSEQ_LOCAL && sc.diff > 0) {
-        set_last_error("batch local alignment needs diff <= 0 (padded columns must not outscore real ones)");
-        return ANYSEQ_ERR_UNSUPPORTED;
-    }
+    rc = batch_prologue(sc, b.npairs, &sp, &affine, out);
+    if (rc || b.npairs == 0) return rc;
     ANYSEQ_CUDA_CHECK(cudaEventRecord(ev0_, stream_));
-    int max_long, max_short;
-    int launches = 1;
-    if (!b.q_len && !b.s_len) {
-        max_long = std::max(b.q_len_uniform, b.s_len_uniform);
-        max_short = std::min(b.q_len_uniform, b.s_len_uniform);
-    } else {
-        int* d_stats = misc_.as<int>() + kMiscOut;
-        ANYSEQ_CUDA_CHECK(cudaMemsetAsync(d_stats, 0, sizeof(int) * 2, stream_));
-        batch_len_stats_kernel<<<(int)std::min<long long>(sm_count * 8, (b.npairs + 255) / 256), 256, 0, stream_>>>(
-            b.q_len, b.s_len, b.q_len_uniform, b.s_len_uniform, b.npairs, d_stats);
-        ANYSEQ_CUDA_CHECK(cudaGetLastError());
-        ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(h_misc_ + kMiscOut, d_stats, sizeof(int) * 2, cudaMemcpyDeviceToHost, stream_));
-        ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
-        max_long = h_misc_[kMiscOut];
-        max_short = h_misc_[kMiscOut + 1];
-        launches += 1;
-    }
-    use_mask_ = true;     // four symbols: always the column-mask kernels
-    ncodes_ = 5;
-    if (lut_.ensure(512 + 64 + 16)) return ANYSEQ_ERR_NO_DEVICE;
     BatchArgs ba;
     fill_args(ba, b, d_scores);
-    rc = launch_batch(sc, sp, affine, ba, max_long, max_short, stream_);
-    if (rc) return rc;
-    ANYSEQ_CUDA_CHECK(cudaEventRecord(ev1_, stream_));
-    ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
-    float ms = 0.f;
-    ANYSEQ_CUDA_CHECK(cudaEventElapsedTime(&ms, ev0_, ev1_));
-    if (out) { out->kernel_ms = ms; out->kernel_launches = launches; }
-    return ANYSEQ_OK;
+    int max_long = std::max(b.q_len_uniform, b.s_len_uniform), max_short = std::min(b.q_len_uniform, b.s_len_uniform);
+    int launches = 1;
+    if (b.q_len || b.s_len) {
+        if ((rc = batch_len_stats(ba, &max_long, &max_short))) return rc;
+        launches += 1;
+    }
+    if ((rc = use_2bit_alphabet())) return rc;
+    if ((rc = launch_batch(sc, sp, affine, ba, max_long, max_short, stream_))) return rc;
+    return batch_epilogue(launches, out);
 }
 
 int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_packed_batch& b, int32_t* scores,
@@ -121,17 +88,11 @@ int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_pack
     ANYSEQ_CUDA_CHECK(cudaSetDevice(device));
     ScoreParams sp;
     bool affine;
-    int rc = make_score_params(sc, &sp, &affine);
+    int rc = check_packed_batch(b, scores);
     if (rc) return rc;
-    if ((rc = check_packed_batch(b))) return rc;
-    if (out) { std::memset(out, 0, sizeof(*out)); out->end_i = out->end_j = -1; }
     const int64_t np = b.npairs;
-    if (np == 0) return ANYSEQ_OK;
-    if (!scores) { set_last_error("packed batch: null score array"); return ANYSEQ_ERR_BAD_ARG; }
-    if (sc.mode == ANYSEQ_LOCAL && sc.diff > 0) {
-        set_last_error("batch local alignment needs diff <= 0 (padded columns must not outscore real ones)");
-        return ANYSEQ_ERR_UNSUPPORTED;
-    }
+    rc = batch_prologue(sc, np, &sp, &affine, out);
+    if (rc || np == 0) return rc;
     // length statistics + byte extent of every sequence array (host pass over the metadata only)
     auto qlen = [&](int64_t p) { return b.q_len ? b.q_len[p] : b.q_len_uniform; };
     auto slen = [&](int64_t p) { return b.s_len ? b.s_len[p] : b.s_len_uniform; };
@@ -157,9 +118,7 @@ int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_pack
             }
         }
     }
-    use_mask_ = true;
-    ncodes_ = 5;
-    if (lut_.ensure(512 + 64 + 16)) return ANYSEQ_ERR_NO_DEVICE;
+    if ((rc = use_2bit_alphabet())) return rc;
     if (!copy_stream_) {
         ANYSEQ_CUDA_CHECK(cudaStreamCreateWithFlags(&copy_stream_, cudaStreamNonBlocking));
         for (int i = 0; i < 2; ++i) {
@@ -229,17 +188,9 @@ int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_pack
         ANYSEQ_CUDA_CHECK(cudaEventRecord(p2_done_[slot], stream_));
         launches += 1;
     }
-    ANYSEQ_CUDA_CHECK(cudaEventRecord(ev1_, stream_));
+    rc = batch_epilogue(launches, out);
     ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(copy_stream_));
-    ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
-    float ms = 0.f;
-    ANYSEQ_CUDA_CHECK(cudaEventElapsedTime(&ms, ev0_, ev1_));
-    if (out) {
-        out->kernel_ms = ms;
-        out->kernel_launches = launches;
-
-    }
-    return ANYSEQ_OK;
+    return rc;
 }
 
 }  // namespace anyseq

@@ -290,12 +290,10 @@ static void parallel_copy(char* dst, const char* src, size_t n, int threads)
 int Engine::score_batch_host(const anyseq_scoring& sc, const char* q, const int64_t* qoff, const char* s,
                              const int64_t* soff, int64_t npairs, int32_t* scores, anyseq_result* out)
 {
-    if (out) { std::memset(out, 0, sizeof(*out)); out->end_i = out->end_j = -1; }
-    if (npairs == 0) return ANYSEQ_OK;
     ScoreParams sp;
     bool affine;
-    int rc = make_score_params(sc, &sp, &affine);
-    if (rc) return rc;
+    int rc = batch_prologue(sc, npairs, &sp, &affine, out);
+    if (rc || npairs == 0) return rc;
     // chunk = up to 64 MiB of packed symbols; a single pair is at most ~2 GiB, far above any slot, so the
     // slot capacity follows the largest pair when one exceeds the default
     const int64_t total = (qoff[npairs] - qoff[0]) + (soff[npairs] - soff[0]);

@@ -158,6 +158,12 @@ private:
     int balance_warps(int nb, int max_h, long long strips_total, int K, bool chained) const;
     int launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool affine, BatchArgs& ba, int max_long,
                      int max_short, cudaStream_t st);
+    // batch.cu: max over pairs of the longer and of the shorter length (synchronises stream_)
+    int batch_len_stats(const BatchArgs& ba, int* max_long, int* max_short);
+    // batch.cu: ends a timed batch call on stream_ (ev0_ .. ev1_) and reports the time and launch count in *out
+    int batch_epilogue(int launches, anyseq_result* out);
+    // batch_packed2.cu: 2-bit input has codes 1..4 (0 matches nothing) and always runs the column-mask kernels
+    int use_2bit_alphabet();
 
     cudaStream_t stream_ = nullptr;
     cudaEvent_t ev0_ = nullptr, ev1_ = nullptr;
@@ -193,6 +199,9 @@ private:
 
 void set_last_error(const std::string& s);
 int make_score_params(const anyseq_scoring& sc, ScoreParams* sp, bool* affine);
+// batch.cu: the checks every batch entry point starts with -- the scheme, a cleared *out, and local alignment with
+// diff > 0 refused for a non-empty batch (padded columns must not outscore real ones)
+int batch_prologue(const anyseq_scoring& sc, int64_t npairs, ScoreParams* sp, bool* affine, anyseq_result* out);
 
 }  // namespace anyseq
 

@@ -804,6 +804,54 @@ def test_batch_packed_16bit_kernels(aligner, oracle):
                     assert got[p] == want, (lq, ls, mode, sch, p)
 
 
+@pytest.mark.parametrize("npairs", [201, 202, 203])
+def test_batch_packed_16bit_kernels_ragged(aligner, oracle, npairs):
+    """ragged DNA pairs of at most 512 symbols (four pairs per warp): neighbours of unequal shape, runs of equal
+    shape, empty and 1-symbol sequences in both half-warps of the first item, a last item with 1-3 pairs; four and
+    two pairs per warp and the 32-bit kernel must agree with each other and with the oracle on every pair"""
+    import anyseq_b200 as A
+    rng = np.random.default_rng(npairs)
+    special = [(0, 37), (1, 0), (0, 0), (1, 1), (150, 0), (1, 512), (0, 1), (512, 1)]     # (lq, ls) of pairs 0..7
+    qs, ss = [], []
+    for p in range(npairs):
+        if p < len(special):
+            lq, ls = special[p]
+        elif p % 5 == 4:
+            lq, ls = len(qs[-1]), len(ss[-1])            # same shape as the previous pair
+        else:
+            lq = int(rng.integers(2, 201)); ls = int(rng.integers(2, 513))
+            if p % 7 == 0:
+                lq, ls = ls, lq
+        q = _rand(rng, lq); s = _rand(rng, ls)
+        k = min(lq, ls)
+        if k and p % 3:
+            o = int(rng.integers(0, ls - k + 1))
+            s[o:o + k] = q[:k]
+            s[rng.integers(0, ls, max(1, ls // 15))] = ACGT[p % 4]
+        qs.append(q); ss.append(s)
+    qd, qo = _pack(qs); sd, so = _pack(ss)
+    for sch in (A.linear_scoring_scheme(2, -1, -1), A.affine_scoring_scheme(2, -1, -2, -1), A.affine_scoring_scheme(5, -4, -10, -1)):
+        for mode in MODES:
+            aligner.set_option("batch_packed", 1)
+            quad, _ = aligner.score_batch(mode, qd, qo, sd, so, sch)
+            aligner.set_option("batch_quad", 0)
+            x2, _ = aligner.score_batch(mode, qd, qo, sd, so, sch)
+            aligner.set_option("batch_quad", 1)
+            aligner.set_option("batch_packed", 0)
+            ref, _ = aligner.score_batch(mode, qd, qo, sd, so, sch)
+            aligner.set_option("batch_packed", 1)
+            assert (quad == x2).all(), (npairs, mode, sch, np.flatnonzero(quad != x2)[:5])
+            assert (quad == ref).all(), (npairs, mode, sch, np.flatnonzero(quad != ref)[:5])
+            for p, (q, s) in enumerate(zip(qs, ss)):
+                if len(q) == 0 or len(s) == 0:
+                    want = aligner.score(mode, q, s, sch).score      # quirk Q12 values, same as the single-pair path
+                elif sch.affine:
+                    want = oracle.textbook_affine(mode, q, s, sch.same, sch.diff, sch.gap_init, sch.gap_extend)
+                else:
+                    want = oracle.textbook_linear(mode, q, s, sch.same, sch.diff, sch.gap_extend)
+                assert ref[p] == want, (npairs, mode, sch, p, len(q), len(s))
+
+
 def test_batch_packed2_vs_oracle_and_byte_path(aligner, oracle):
     """anyseq_score_batch_packed2 (2-bit packed DNA, BASELINE configs[3] shape and ragged shapes): host pipeline and
     device-resident entry, uniform strides and explicit offsets/lengths, all schemes -- scores must equal the byte
