@@ -5,7 +5,7 @@ The package holds only what the path needs: ``csrc/`` (CUDA kernels + C ABI),
 (the host-side mirror of the reference's operator surface).
 """
 from .api import (  # noqa: F401
-    Aligner, AlignmentResult, BatchStream, ScoringScheme, REFERENCE_SCORING,
+    Aligner, AlignmentResult, BatchAlignment, BatchStream, ScoringScheme, REFERENCE_SCORING,
     affine_scoring_scheme, linear_scoring_scheme, cigar, default_aligner, pack2, plan_launch,
     global_alignment_score, semiglobal_alignment_score, local_alignment_score,
     construct_global_alignment, construct_semiglobal_alignment, construct_local_alignment,

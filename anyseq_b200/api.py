@@ -70,6 +70,28 @@ def cigar(aligned_query: bytes, aligned_subject: bytes) -> str:
     return buf.raw[:n].decode("ascii")
 
 
+@dataclass
+class BatchAlignment:
+    """Full-matrix tracebacks of a batch (``Aligner.align_batch``): per pair p the score, end cell
+    (get_score_pos()), start cell (get_alignment_start()) and aligned rows anyseq_align_full gives for it."""
+    scores: np.ndarray              # (npairs,) int32
+    ends: np.ndarray                # (npairs, 2) int32
+    starts: np.ndarray              # (npairs, 2) int32
+    aligned_query: np.ndarray       # uint8, pair p at offsets[p] .. offsets[p] + lq + ls
+    aligned_subject: np.ndarray
+    offsets: np.ndarray             # (npairs + 1,) int64: (q_off[p] - q_off[0]) + (s_off[p] - s_off[0])
+    kernel_ms: float = 0.0
+    kernel_launches: int = 0
+
+    def alignment(self, p: int):
+        """(aligned_query, aligned_subject) of pair p as bytes"""
+        a, b = int(self.offsets[p]), int(self.offsets[p + 1])
+        return self.aligned_query[a:b].tobytes(), self.aligned_subject[a:b].tobytes()
+
+    def cigar(self, p: int) -> str:
+        return cigar(*self.alignment(p))
+
+
 class Aligner:
     """One engine per (process, GPU): wraps an ``anyseq_ctx``."""
 
@@ -199,6 +221,44 @@ class Aligner:
                                                         C.c_void_p(d_q_off), C.c_void_p(d_subjects),
                                                         C.c_void_p(d_s_off), npairs, C.c_void_p(d_scores),
                                                         C.byref(res)))
+        return AlignmentResult(res.score, -1, -1, res.kernel_ms, res.kernel_launches)
+
+    # -- full-matrix tracebacks of batches (anyseq_align_batch) --------------
+    def align_batch(self, mode, queries, q_off, subjects, s_off, scoring: ScoringScheme = REFERENCE_SCORING) -> BatchAlignment:
+        """traceback_full of every pair (as align_full) in one launch; every subject <= 1024 symbols"""
+        q, s = as_u8(queries), as_u8(subjects)
+        qo = np.ascontiguousarray(q_off, dtype=np.int64)
+        so = np.ascontiguousarray(s_off, dtype=np.int64)
+        npairs = len(qo) - 1
+        offsets = (qo - qo[0]) + (so - so[0])
+        total = int(offsets[-1])
+        scores = np.zeros(max(npairs, 1), dtype=np.int32)
+        ends = np.zeros((max(npairs, 1), 2), dtype=np.int32)
+        starts = np.zeros((max(npairs, 1), 2), dtype=np.int32)
+        oq = np.zeros(max(total, 1), dtype=np.uint8)
+        os_ = np.zeros(max(total, 1), dtype=np.uint8)
+        sc = make_scoring(mode, scoring.same, scoring.diff, scoring.gap_init, scoring.gap_extend)
+        res = Result()
+        i64p = C.POINTER(C.c_int64)
+        self._check(self._lib.anyseq_align_batch(self._ctx, C.byref(sc), capi._ptr(q), qo.ctypes.data_as(i64p),
+                                                 capi._ptr(s), so.ctypes.data_as(i64p), npairs, capi._ptr(scores),
+                                                 capi._ptr(ends), capi._ptr(starts), capi._ptr(oq), capi._ptr(os_),
+                                                 C.byref(res)))
+        return BatchAlignment(scores[:npairs], ends[:npairs], starts[:npairs], oq[:total], os_[:total], offsets,
+                              res.kernel_ms, res.kernel_launches)
+
+    def align_batch_device(self, mode, d_queries: int, d_q_off: int, d_subjects: int, d_s_off: int, npairs: int,
+                           d_scores: int, d_ends: int, d_starts: int, d_aligned_query: int, d_aligned_subject: int,
+                           scoring: ScoringScheme = REFERENCE_SCORING) -> AlignmentResult:
+        """align_batch on device memory (raw pointers; d_ends / d_starts may be 0): the aligned rows of pair p start at
+        (q_off[p] - q_off[0]) + (s_off[p] - s_off[0])"""
+        sc = make_scoring(mode, scoring.same, scoring.diff, scoring.gap_init, scoring.gap_extend)
+        res = Result()
+        vp = C.c_void_p
+        self._check(self._lib.anyseq_align_batch_device(self._ctx, C.byref(sc), vp(d_queries), vp(d_q_off),
+                                                        vp(d_subjects), vp(d_s_off), npairs, vp(d_scores),
+                                                        vp(d_ends or None), vp(d_starts or None), vp(d_aligned_query),
+                                                        vp(d_aligned_subject), C.byref(res)))
         return AlignmentResult(res.score, -1, -1, res.kernel_ms, res.kernel_launches)
 
     # -- 2-bit packed DNA batches (anyseq_score_batch_packed2) -----------------

@@ -16,11 +16,11 @@ OUT = os.environ.get("ANYSEQ_BUILD_DIR") or os.path.join(_HERE, "_build")   # AN
 LIB = os.path.join(OUT, "libanyseq_b200.so")
 CLI = os.path.join(OUT, "align")
 
-LIB_SOURCES = ["engine.cu", "capi.cu", "microbench.cu", "inbox.cu", "traceback.cu", "traceback_full.cu", "batch.cu", "batch_x2.cu", "batch_stream.cu", "batch_packed2.cu",
+LIB_SOURCES = ["engine.cu", "capi.cu", "microbench.cu", "inbox.cu", "traceback.cu", "traceback_full.cu", "batch.cu", "batch_x2.cu", "batch_stream.cu", "batch_packed2.cu", "batch_align.cu",
                "strip_inst_00.cu", "strip_inst_01.cu", "strip_inst_10.cu", "strip_inst_11.cu",
                "strip_inst_10t.cu", "strip_inst_11t.cu", "strip_inst_01p.cu"]
 CLI_SOURCES = ["align_main.cpp", "sequence_io.cpp", "alignment_io.cpp"]
-HEADERS = ["common.cuh", "engine.cuh", "strip_kernel.cuh", "strip_packed.cuh", "strip_inst.inl", "batch.cuh", "sequence_io.h", "alignment_io.h",
+HEADERS = ["common.cuh", "engine.cuh", "strip_kernel.cuh", "strip_packed.cuh", "strip_inst.inl", "batch.cuh", "traceback_full.cuh", "sequence_io.h", "alignment_io.h",
            os.path.join("..", "..", "include", "anyseq.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

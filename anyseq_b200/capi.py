@@ -23,7 +23,7 @@ EXPORTED_SYMBOLS = [
     "global_alignment_score", "semiglobal_alignment_score", "local_alignment_score",
     "construct_global_alignment", "construct_semiglobal_alignment", "construct_local_alignment",
     "construct_global_alignment_fulltb", "construct_semiglobal_alignment_fulltb", "construct_local_alignment_fulltb",
-    "anyseq_align_full", "anyseq_align_sharded",
+    "anyseq_align_full", "anyseq_align_sharded", "anyseq_align_batch", "anyseq_align_batch_device",
     "anyseq_ctx_create", "anyseq_ctx_destroy", "anyseq_last_error", "anyseq_ctx_tune", "anyseq_ctx_set_option",
     "anyseq_score", "anyseq_score_device", "anyseq_align", "anyseq_last_splits", "anyseq_last_split_types", "anyseq_cigar",
     "anyseq_score_batch", "anyseq_score_batch_device",
@@ -130,6 +130,12 @@ def load_library(path: str | None = None):
     L.anyseq_align_full.restype = C.c_int
     L.anyseq_align_full.argtypes = [vp, C.POINTER(Scoring), vp, C.c_int, vp, C.c_int, vp, vp, C.POINTER(Result),
                                     C.POINTER(C.c_int32)]
+    L.anyseq_align_batch.restype = C.c_int
+    L.anyseq_align_batch.argtypes = [vp, C.POINTER(Scoring), vp, i64p, vp, i64p, C.c_int64, vp, vp, vp, vp, vp,
+                                     C.POINTER(Result)]
+    L.anyseq_align_batch_device.restype = C.c_int
+    L.anyseq_align_batch_device.argtypes = [vp, C.POINTER(Scoring), vp, vp, vp, vp, C.c_int64, vp, vp, vp, vp, vp,
+                                            C.POINTER(Result)]
     L.anyseq_last_splits.restype = C.c_int
     L.anyseq_last_splits.argtypes = [vp, C.POINTER(C.c_int32), C.c_int]
     L.anyseq_last_split_types.restype = C.c_int

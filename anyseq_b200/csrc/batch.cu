@@ -21,21 +21,31 @@
 
 namespace anyseq {
 
-// stats[0] = max over pairs of max(lenq, lens), stats[1] = max over pairs of min(lenq, lens), clamped to 2^31 - 1
+// stats[0] = max over pairs of max(lenq, lens), stats[1] = max over pairs of min(lenq, lens), stats[2] / stats[3] = max
+// over pairs of lenq / lens, clamped to 2^31 - 1; stats[4] = 1 when a pair has a negative length (decreasing offsets)
 __global__ void batch_stats_kernel(const BatchArgs a, int* __restrict__ stats)
 {
-    int mx = 0, mn = 0;
+    int mx = 0, mn = 0, mq = 0, ms = 0, neg = 0;
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < a.npairs; p += (long long)gridDim.x * blockDim.x) {
         const long long lq = batch_q_len(a, p), ls = batch_s_len(a, p);
         const long long hi = lq > ls ? lq : ls, lo = lq > ls ? ls : lq;
         mx = max(mx, (int)min(hi, (long long)0x7fffffff));
         mn = max(mn, (int)min(lo, (long long)0x7fffffff));
+        mq = max(mq, (int)min(lq, (long long)0x7fffffff));
+        ms = max(ms, (int)min(ls, (long long)0x7fffffff));
+        neg |= lo < 0;
     }
     for (int o = 16; o > 0; o >>= 1) {
         mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
         mn = max(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        mq = max(mq, __shfl_xor_sync(0xffffffffu, mq, o));
+        ms = max(ms, __shfl_xor_sync(0xffffffffu, ms, o));
+        neg |= __shfl_xor_sync(0xffffffffu, neg, o);
     }
-    if ((threadIdx.x & 31) == 0) { atomicMax(&stats[0], mx); atomicMax(&stats[1], mn); }
+    if ((threadIdx.x & 31) == 0) {
+        atomicMax(&stats[0], mx); atomicMax(&stats[1], mn); atomicMax(&stats[2], mq); atomicMax(&stats[3], ms);
+        if (neg) stats[4] = 1;
+    }
 }
 
 template <int MODE, bool AFFINE, int K, bool MASK>
@@ -290,16 +300,19 @@ int batch_prologue(const anyseq_scoring& sc, int64_t npairs, ScoreParams* sp, bo
     return ANYSEQ_OK;
 }
 
-int Engine::batch_len_stats(const BatchArgs& ba, int* max_long, int* max_short)
+int Engine::batch_len_stats(const BatchArgs& ba, int* max_long, int* max_short, int* max_q, int* max_s, bool* negative)
 {
     int* d_stats = misc_.as<int>() + kMiscOut;
-    ANYSEQ_CUDA_CHECK(cudaMemsetAsync(d_stats, 0, sizeof(int) * 2, stream_));
+    ANYSEQ_CUDA_CHECK(cudaMemsetAsync(d_stats, 0, sizeof(int) * 5, stream_));
     batch_stats_kernel<<<(int)std::min<long long>(sm_count * 8, (ba.npairs + 255) / 256), 256, 0, stream_>>>(ba, d_stats);
     ANYSEQ_CUDA_CHECK(cudaGetLastError());
-    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(h_misc_ + kMiscOut, d_stats, sizeof(int) * 2, cudaMemcpyDeviceToHost, stream_));
+    ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(h_misc_ + kMiscOut, d_stats, sizeof(int) * 5, cudaMemcpyDeviceToHost, stream_));
     ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(stream_));
     *max_long = h_misc_[kMiscOut];
     *max_short = h_misc_[kMiscOut + 1];
+    if (max_q) *max_q = h_misc_[kMiscOut + 2];
+    if (max_s) *max_s = h_misc_[kMiscOut + 3];
+    if (negative) *negative = h_misc_[kMiscOut + 4] != 0;
     return ANYSEQ_OK;
 }
 

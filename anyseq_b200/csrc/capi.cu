@@ -122,6 +122,27 @@ int anyseq_align_full(anyseq_ctx* ctx, const anyseq_scoring* sc, const char* que
     return rc;
 }
 
+int anyseq_align_batch(anyseq_ctx* ctx, const anyseq_scoring* sc, const char* queries, const int64_t* q_off,
+                       const char* subjects, const int64_t* s_off, int64_t npairs, int32_t* scores,
+                       int32_t* ends, int32_t* starts, char* alQuery, char* alSubject, anyseq_result* out)
+{
+    if (!ctx || !sc) return ANYSEQ_ERR_BAD_ARG;
+    return ctx->eng.align_batch_host(*sc, queries, q_off, subjects, s_off, npairs, scores, ends, starts, alQuery,
+                                     alSubject, out);
+}
+
+int anyseq_align_batch_device(anyseq_ctx* ctx, const anyseq_scoring* sc, const void* d_queries,
+                              const int64_t* d_q_off, const void* d_subjects, const int64_t* d_s_off,
+                              int64_t npairs, int32_t* d_scores, int32_t* d_ends, int32_t* d_starts,
+                              char* d_alQuery, char* d_alSubject, anyseq_result* out)
+{
+    if (!ctx || !sc || npairs < 0 || (npairs > 0 && (!d_q_off || !d_s_off || !d_scores || !d_alQuery || !d_alSubject)))
+        return ANYSEQ_ERR_BAD_ARG;
+    return ctx->eng.align_batch_device(*sc, static_cast<const uint8_t*>(d_queries), d_q_off,
+                                       static_cast<const uint8_t*>(d_subjects), d_s_off, npairs, d_scores, d_ends,
+                                       d_starts, d_alQuery, d_alSubject, out);
+}
+
 int anyseq_last_splits(anyseq_ctx* ctx, int32_t* out, int cap)
 {
     if (!ctx) return ANYSEQ_ERR_BAD_ARG;

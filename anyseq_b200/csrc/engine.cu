@@ -379,7 +379,7 @@ void Engine::destroy()
     if (device >= 0) cudaSetDevice(device);
     DeviceBuffer* bufs[] = {&seq_q_, &seq_s_, &seq_qr_, &seq_sr_, &col_, &rowH_, &rowF_, &corner_,
                             &progress_, &jobs_, &misc_, &lut_, &col2_, &aux_, &aux2_, &pred_,
-                            &tb_out_, &blockmax_, &edges_, &multi_, &p2_[0], &p2_[1]};
+                            &tb_out_, &blockmax_, &edges_, &multi_, &p2_[0], &p2_[1], &batch_pred_, &batch_io_};
     drop_host_batch_stream();
     for (DeviceBuffer* b : bufs) b->release();
     if (h_misc_) cudaFreeHost(h_misc_);

@@ -121,6 +121,14 @@ public:
     int score_batch_host(const anyseq_scoring& sc, const char* q, const int64_t* qoff,
                          const char* s, const int64_t* soff, int64_t npairs, int32_t* scores,
                          anyseq_result* out);
+    // full-matrix tracebacks of a batch of pairs with subjects of at most 1024 symbols (batch_align.cu): per pair what
+    // align_full_host gives; ends / starts may be null
+    int align_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, const int64_t* d_qoff, const uint8_t* d_s,
+                           const int64_t* d_soff, int64_t npairs, int32_t* d_scores, int32_t* d_ends, int32_t* d_starts,
+                           char* d_alq, char* d_als, anyseq_result* out);
+    int align_batch_host(const anyseq_scoring& sc, const char* q, const int64_t* qoff, const char* s, const int64_t* soff,
+                         int64_t npairs, int32_t* scores, int32_t* ends, int32_t* starts, char* alq, char* als,
+                         anyseq_result* out);
     // 2-bit packed DNA batches (batch_packed2.cu)
     int score_batch_packed2_device(const anyseq_scoring& sc, const anyseq_packed_batch& b, int32_t* d_scores,
                                    anyseq_result* out);
@@ -158,8 +166,10 @@ private:
     int balance_warps(int nb, int max_h, long long strips_total, int K, bool chained) const;
     int launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool affine, BatchArgs& ba, int max_long,
                      int max_short, cudaStream_t st);
-    // batch.cu: max over pairs of the longer and of the shorter length (synchronises stream_)
-    int batch_len_stats(const BatchArgs& ba, int* max_long, int* max_short);
+    // batch.cu: max over pairs of the longer and of the shorter length, optionally of the query and of the subject
+    // length and whether some pair has a negative length (synchronises stream_)
+    int batch_len_stats(const BatchArgs& ba, int* max_long, int* max_short, int* max_q = nullptr, int* max_s = nullptr,
+                        bool* negative = nullptr);
     // batch.cu: ends a timed batch call on stream_ (ev0_ .. ev1_) and reports the time and launch count in *out
     int batch_epilogue(int launches, anyseq_result* out);
     // batch_packed2.cu: 2-bit input has codes 1..4 (0 matches nothing) and always runs the column-mask kernels
@@ -177,6 +187,8 @@ private:
     DeviceBuffer edges_;         // full-matrix traceback: right edge column (H, E) of every 128-column strip
     DeviceBuffer blockmax_;      // local end-cell tracking: one key per 1024 x 1024 reference block
     DeviceBuffer p2_[2];         // packed2 host pipeline: two device chunk slots
+    DeviceBuffer batch_pred_;    // batch tracebacks: one predecessor slab per resident warp
+    DeviceBuffer batch_io_;      // batch tracebacks from host memory: inputs and outputs on the device
     cudaStream_t copy_stream_ = nullptr;                     // packed2 host pipeline: H2D of chunk c+1 under the kernel of chunk c
     cudaEvent_t p2_ready_[2] = {nullptr, nullptr}, p2_done_[2] = {nullptr, nullptr};
     int* h_misc_ = nullptr;           // pinned mirror of misc_

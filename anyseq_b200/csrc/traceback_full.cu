@@ -16,6 +16,7 @@
 //      (H(i,j-1) >= E(i,j-1)), so the walk and the tie order NO_GAP > GAP_Q > GAP_S are the reference's.
 // The Gotoh variant is build-defined like every affine entry point (parity unpinned vs the reference).
 #include "engine.cuh"
+#include "traceback_full.cuh"
 
 #include <algorithm>
 #include <cstring>
@@ -23,7 +24,6 @@
 namespace anyseq {
 
 constexpr int kFullBlockW = 128;
-enum : int { kFSrcNone = 0, kFSrcE = 1, kFSrcF = 2, kFSrcDiag = 3 };   // src/align.impala:37-40
 
 // pred16[i * pitch + b * 32 + lane] = 4 cells x 4 bits of row i, columns 128 b + 4 lane ...
 __global__ void __launch_bounds__(128)
@@ -73,22 +73,9 @@ fulltb_dp_kernel(const uint8_t* __restrict__ q, const uint8_t* __restrict__ s, i
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
                 const int up = H[c];
-                int eext = 0, fext = 0;
-                int eo = lft + go;
-                if (e + ge > eo) { eo = e + ge; eext = 1; }
-                e = eo;
-                int fo = up + go;
-                if (F[c] + ge > fo) { fo = F[c] + ge; fext = 1; }
-                int score = d + ((qc == sc[c]) ? same : diff);
-                int src = kFSrcDiag;
-                if (e > score) { score = e; src = kFSrcE; }
-                if (fo > score) { score = fo; src = kFSrcF; }
-                if (local && 0 > score) { score = 0; src = kFSrcNone; }
-                bits |= (unsigned)(src | (eext << 2) | (fext << 3)) << (4 * c);
+                bits |= fulltb_cell(d + ((qc == sc[c]) ? same : diff), up, lft, e, F[c], go, ge, local) << (4 * c);
                 d = up;
-                H[c] = score;
-                F[c] = fo;
-                lft = score;
+                H[c] = lft;
             }
             hr = lft;
             er = e;
@@ -118,18 +105,7 @@ __global__ void fulltb_walk_kernel(const uint8_t* __restrict__ q, const uint8_t*
             out_q[pos] = q[i]; out_s[pos] = '_'; --i; continue;
         }
         const unsigned p = (pred16[(size_t)i * pitch + (size_t)(j >> 2)] >> (4 * (j & 3))) & 15u;
-        if (state == 0) {
-            const int src = (int)(p & 3u);
-            if (src == kFSrcNone) break;
-            if (src == kFSrcDiag) { out_q[pos] = q[i]; out_s[pos] = s[j]; --i; --j; }
-            else state = (src == kFSrcE) ? 1 : 2;
-        } else if (state == 1) {
-            out_q[pos] = '_'; out_s[pos] = s[j];
-            state = ((p >> 2) & 1u) ? 1 : 0; --j;
-        } else {
-            out_q[pos] = q[i]; out_s[pos] = '_';
-            state = ((p >> 3) & 1u) ? 2 : 0; --i;
-        }
+        if (!fulltb_walk_step(p, i, j, state, q[i], s[j], out_q, out_s)) break;
     }
     start[0] = i + 1;
     start[1] = j + 1;

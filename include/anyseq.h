@@ -175,6 +175,23 @@ int anyseq_align_full(anyseq_ctx* ctx, const anyseq_scoring* sc,
                       const char* query, int lenq, const char* subject, int lens,
                       char* alQuery, char* alSubject, anyseq_result* out, int32_t* start);
 
+/* Full-matrix traceback of a batch of independent pairs (traceback_full per pair, as anyseq_align_full).
+ * Pair p is queries[q_off[p] .. q_off[p+1]) vs subjects[s_off[p] .. s_off[p+1]); every subject <= 1024 symbols.
+ * Pair p's aligned rows occupy alQuery/alSubject[o_p .. o_p + lq + ls) with
+ * o_p = (q_off[p] - q_off[0]) + (s_off[p] - s_off[0]), i.e. both buffers hold
+ * (q_off[npairs] - q_off[0]) + (s_off[npairs] - s_off[0]) bytes.
+ * scores[npairs]; ends[2*npairs] = get_score_pos(), starts[2*npairs] = get_alignment_start() (either may be NULL).
+ * Pairs are not transposed.  ANYSEQ_ERR_UNSUPPORTED for a subject longer than 1024 (use anyseq_align_full) and
+ * when the batch's scratch or outputs do not fit in device memory (split the batch); ANYSEQ_ERR_BAD_ARG for
+ * decreasing offsets.  The _device variant takes device pointers for every array. */
+int anyseq_align_batch(anyseq_ctx* ctx, const anyseq_scoring* sc, const char* queries, const int64_t* q_off,
+                       const char* subjects, const int64_t* s_off, int64_t npairs, int32_t* scores,
+                       int32_t* ends, int32_t* starts, char* alQuery, char* alSubject, anyseq_result* out);
+int anyseq_align_batch_device(anyseq_ctx* ctx, const anyseq_scoring* sc, const void* d_queries,
+                              const int64_t* d_q_off, const void* d_subjects, const int64_t* d_s_off,
+                              int64_t npairs, int32_t* d_scores, int32_t* d_ends, int32_t* d_starts,
+                              char* d_alQuery, char* d_alSubject, anyseq_result* out);
+
 /* Derived view of an alignment pair: CIGAR string (=/X/I/D run-length, I = gap
  * in the query ('_' in alQuery), D = gap in the subject), skipping blank
  * columns.  Returns the length written (excluding the NUL) or -needed if cap is
