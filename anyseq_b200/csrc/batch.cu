@@ -158,7 +158,7 @@ __global__ void __launch_bounds__(kThreads, (K >= 32 ? 4 : (K >= 16 ? 5 : 6))) b
                         dcarry = xl;
                         st.xleft = xl;
                         st.e = el;
-                        Cell<LOCAL, AFFINE, K, false, MASK, 1, 0, 0>::run(X, F, sc, st, k);
+                        Cell<LOCAL, AFFINE, K, false, MASK, 1, 0, 0, true>::run(X, F, sc, st, k);    // coupled cells
                         hr = st.xleft;
                         er = st.e;
                         if constexpr (MODE == kSemiglobal) {

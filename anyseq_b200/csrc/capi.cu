@@ -71,7 +71,10 @@ int anyseq_ctx_set_option(anyseq_ctx* ctx, const char* name, int value)
         t.watchdog_ms = value;
     }
     else if (n == "band_slack" && value >= 1) t.band_slack = value;
-    else if (n == "cell_form" && value >= -1 && value <= 2) t.cell_form = value;
+    else if (n == "cell_form") {
+        if (value != -1 && value != 1 && value != 2) { set_last_error("cell_form must be -1, 1 or 2"); return ANYSEQ_ERR_BAD_ARG; }
+        t.cell_form = value;
+    }
     else if (n == "packed_cells" && value >= -1 && value <= 1) t.packed_cells = value;
     else if (n == "force_generic") t.force_generic = value != 0;
     else if (n == "force_affine") t.force_affine = value != 0;

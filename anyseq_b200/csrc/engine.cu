@@ -179,19 +179,20 @@ static KernelFn pick_kernel(bool local, bool affine, int K, bool mask, bool trac
     return affine ? get_strip_kernel_01(K, mask, form) : get_strip_kernel_00(K, mask, form);
 }
 
-// Cell form of a launch (strip_kernel.cuh: 0 = coupled, 1 = decoupled, 2 = mixed).  Measured on B200s with the warps of a
+// Cell form of a launch (strip_kernel.cuh: 1 = decoupled, 2 = mixed).  Measured on B200s with the warps of a
 // scheduler on adjacent strips, semiglobal Gotoh, GCUPS, coupled / decoupled / mixed: 4.6 Mbp pair, three warps per
 // scheduler: 3853 / 3864-3885 on four different boxes / 3974 on one box, 3753-3758 on three others (local Gotoh:
 // 3315 / 3038 / 3302-3505); 575 k-column slice, two per scheduler: 2846 / 3195 / 3159; lone warps (K = 32 slice):
 // 2214 / 2885 / 2753; 1 Mbp x 1 Mbp: 2500 / 3157 / 2654.  So: the decoupled cells everywhere -- they are the fastest or
 // within 2 % of it and the most repeatable -- except for wide LOCAL Gotoh launches, whose decoupled cell needs one more
-// instruction; those run the mixed cells.
+// instruction; those run the mixed cells.  The coupled cells, never ahead by more than noise, are not built for these
+// kernels.  cell_form 1 / 2 forces a form, any other value picks per launch.
 static int pick_form(const Tuning& tune, bool affine, bool mask, int K, long long strips_total, int sm_count, bool local)
 {
-    const bool has_coupled = affine && mask && K >= 8;
-    if (tune.cell_form == 0 || tune.cell_form == 1) return has_coupled ? tune.cell_form : 1;
-    if (tune.cell_form == 2) return (has_coupled && K >= 16) ? 2 : 1;
-    return (has_coupled && K >= 16 && local && strips_total >= 24LL * sm_count) ? 2 : 1;
+    const bool has_mixed = affine && mask && K >= 16;
+    if (tune.cell_form == 1) return 1;
+    if (tune.cell_form == 2) return has_mixed ? 2 : 1;
+    return (has_mixed && local && strips_total >= 24LL * sm_count) ? 2 : 1;
 }
 
 // Packed cells (strip_packed.cuh) hold a warp's scores as 16-bit halves around a re-centred offset.  With go = gi + ge,
@@ -228,7 +229,7 @@ static int rows_per_step(int K, bool mask, bool track)
 // than strips: at most one warp works on a strip at a time, the others would only
 // poll and add spread to the progress of the busy ones -- which is what the
 // strip-to-strip pipeline is sensitive to (measured: profiles/).
-static int default_blocks_per_sm(int K, bool mask, bool track, int occupancy_max, long long nstrips, int sm_count, int form)
+static int default_blocks_per_sm(int K, bool mask, bool track, int occupancy_max, long long nstrips, int sm_count)
 {
     int nb = occupancy_max;
     if (rows_per_step(K, mask, track) >= 2) {
@@ -241,7 +242,6 @@ static int default_blocks_per_sm(int K, bool mask, bool track, int occupancy_max
         int want = (int)std::max<long long>(1, (nstrips + per_round - 1) / per_round);
         if (want > 1 && nstrips * 10 < (long long)want * per_round * 8) --want;
         nb = std::min(nb, std::min(3, want));
-        (void)form;
     }
     return nb;
 }
@@ -409,7 +409,7 @@ int Engine::resident_warps(int K, bool local, bool affine, long long nstrips)
     KernelFn fn = pick_kernel(local, affine, K, use_mask_, track_ && local, form);
     if (!fn) return 0;
     const bool track = track_ && local;
-    int want = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, use_mask_, track, track ? 6 : 3, nstrips, sm_count, form);
+    int want = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, use_mask_, track, track ? 6 : 3, nstrips, sm_count);
     if (!track) want = std::min(want, kMaxStripWarps / kWarpsPerBlock);
     return fit_blocks_per_sm(fn, track, use_mask_, ncodes_, K, want, form) * kWarpsPerBlock * sm_count;
 }
@@ -568,7 +568,7 @@ int Engine::plan_launch(int sms, int mode, bool affine, int m, int n, bool chain
     const int K = pick_K(n, chained, chained ? 0 : m, affine);
     const long long strips = ((long long)n + kWarp * K - 1) / (kWarp * K);
     const int form = pick_form(tune, affine, true, K, strips, sms, local);
-    int nb = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, true, false, 3, strips, sms, form);
+    int nb = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, true, false, 3, strips, sms);
     nb = std::max(1, std::min(nb, kMaxStripWarps / kWarpsPerBlock));
     nb = balance_warps(nb, m, strips, K, chained);
     const int resident = nb * kWarpsPerBlock * sms;
@@ -612,7 +612,7 @@ int Engine::run_jobs(std::vector<Job>& jobs, const ScoreParams& sp, bool local, 
     const int form = packed ? 3 : pick_form(tune, affine, use_mask_, K, strips_total, sm_count, local);
     KernelFn fn = pick_kernel(local, affine, K, use_mask_, track_ && local, form);
     if (!fn) { set_last_error("unsupported columns-per-lane"); return ANYSEQ_ERR_BAD_ARG; }
-    int want = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, use_mask_, track, track ? 6 : 3, strips_total, sm_count, form);
+    int want = tune.blocks_per_sm > 0 ? tune.blocks_per_sm : default_blocks_per_sm(K, use_mask_, track, track ? 6 : 3, strips_total, sm_count);
     if (!track) want = balance_warps(std::min(want, kMaxStripWarps / kWarpsPerBlock), max_h, strips_total, K, chained);
     const int nb = fit_blocks_per_sm(fn, track, use_mask_, ncodes_, K, want, form);
     if (nb < 1) { set_last_error("strip kernel does not fit on an SM"); return ANYSEQ_ERR_UNSUPPORTED; }

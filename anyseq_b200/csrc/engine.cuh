@@ -41,7 +41,7 @@ struct Tuning {
     int band_rows = 0;       // 0 = auto
     int blocks_per_sm = 0;   // 0 = occupancy maximum
     int watchdog_ms = 20000;
-    int cell_form = -1;      // -1 = per launch (engine.cu: pick_form), 0 = coupled, 1 = decoupled cells
+    int cell_form = -1;      // -1 = per launch (engine.cu: pick_form), 1 = decoupled, 2 = mixed cells
     int packed_cells = -1;   // -1 / 1 = packed cells where the score window fits (engine.cu: packed_fits), 0 = never
     int band_slack = 2;      // band height = band_slack * lag * (resident warps) when the strips outnumber the warps
     bool force_generic = false;     // never use the MASK kernels (testing)

@@ -36,20 +36,21 @@
 
 namespace anyseq {
 
-// Cell formulation of the multi-purpose (non-TRACK) kernels:
-//   0  "coupled":   E' = max(E+ge, X_left); H = max3(diag, E', F); X = H+go  -- 3 ALU + 3 FMA ops per Gotoh cell, but the
-//                   loop-carried chain along a row is VIADDMNMX -> VIMNMX3 -> IMAD (about 14 cycles per cell), so a warp
-//                   needs several independent rows or several co-resident warps to fill the issue slots.
-//   1  "decoupled": M = max(F+go, diag) (no horizontal input), E' = max(E+ge, M_left), X = max(E'+go, M)  -- 4 ALU + 2 FMA,
-//                   the loop-carried chain is ONE VIADDMNMX (4 cycles): valid because the E term inside H(i,j-1) can never
-//                   win the maximum that forms E(i,j) (E+go <= E+ge).  A lone warp saturates its scheduler's ALU pipe, so
-//                   half as many (twice as fast) warps are needed -- which is what the strip-to-strip chain, narrow
-//                   problems and multi-GPU slices are sensitive to.
-//   3  "packed":    the decoupled cell on 16-bit halves, two cells per DPX instruction (strip_packed.cuh; global and
-//                   semiglobal Gotoh with column masks, when the scheme's score window fits 16 bits).
-// The forms are built as template parameter FORM of strip_kernel; engine.cu picks per launch: the coupled form where
-// three warps per scheduler can be fed (Gotoh, strips >> warps: 3.71 vs 3.52 TCUPS on the 4.6 Mbp pair), the decoupled
-// form everywhere else (linear gaps, single-band launches, small problems, multi-GPU slices).
+// Cell formulations:
+//   "coupled":   E' = max(E+ge, X_left); H = max3(diag, E', F); X = H+go  -- 3 ALU + 3 FMA ops per Gotoh cell, but the
+//                loop-carried chain along a row is VIADDMNMX -> VIMNMX3 -> IMAD (about 14 cycles per cell), so a warp
+//                needs several independent rows or several co-resident warps to fill the issue slots.
+//   "decoupled": M = max(F+go, diag) (no horizontal input), E' = max(E+ge, M_left), X = max(E'+go, M)  -- 4 ALU + 2 FMA,
+//                the loop-carried chain is ONE VIADDMNMX (4 cycles): valid because the E term inside H(i,j-1) can never
+//                win the maximum that forms E(i,j) (E+go <= E+ge).  A lone warp saturates its scheduler's ALU pipe, so
+//                half as many (twice as fast) warps are needed -- which is what the strip-to-strip chain, narrow
+//                problems and multi-GPU slices are sensitive to.
+// The strip kernels build them as template parameter FORM (engine.cu: pick_form, use_packed):
+//   1  decoupled cells: the default (linear and Gotoh gaps, every strip width).
+//   2  "mixed": even rows coupled, odd rows decoupled -- wide local Gotoh launches (two-row MASK tiles).
+//   3  "packed": the decoupled cell on 16-bit halves, two cells per DPX instruction (strip_packed.cuh) -- global and
+//      semiglobal Gotoh with column masks, when the scheme's score window fits 16 bits.
+// The end-cell tracking kernels (TRACK) run coupled cells: they need H itself to find where the maximum is reached.
 
 constexpr int kWarpsPerBlock = 4;                       // batch kernels, end-cell tracking strip kernels
 constexpr int kThreads = kWarpsPerBlock * kWarp;
@@ -284,10 +285,13 @@ __device__ __forceinline__ int diag_mask_bit(const unsigned (&tm)[W], int r, int
 // The diagonal term of cell C+1 is formed before X[C] is overwritten, so the
 // old value dies in place and no register moves are needed.
 // RS / RO: the row is row RO of an RS-row group (selects its bits in the tile mask).
-// TRACK (local scheme, single-row kernels): also remember WHERE the lane's maximum was first reached, in the
+// COUPLED: the coupled cell (the end-cell tracking strip kernels and the one-pair-per-warp batch kernels), otherwise
+// the decoupled one.
+// TRACK (local scheme, coupled cells): also remember WHERE the lane's maximum was first reached, in the
 // lane's own row-major order (strict '>'), for the reference's end-cell rule (src/scoring_cpu.impala:48-72).
-template <bool LOCAL, bool AFFINE, int K, int PARTIAL, bool MASK, int RS, int RO, int C, bool TRACK = false, int FORM = 0>
+template <bool LOCAL, bool AFFINE, int K, int PARTIAL, bool MASK, int RS, int RO, int C, bool COUPLED, bool TRACK = false>
 struct Cell {
+    static_assert(!TRACK || (LOCAL && COUPLED), "end-cell tracking: local scheme, coupled cells");
     template <int KF, int KS, int W>
     static __device__ __forceinline__ void run(int (&X)[K], int (&F)[KF], const int (&sc)[KS], StepState<W>& s,
                                                const StepConst& k)
@@ -299,7 +303,7 @@ struct Cell {
             if constexpr (MASK) s.dd = diag_plus_sigma_mask<BIT % 32>(s.tm[BIT / 32], up, k.one, k.diff_o, k.same_o);
             else s.dd = diag_plus_sigma(s.qc, sc[C + 1], up, k.one, k.diff_o, k.same_o);
         }
-        if constexpr (FORM == 1) {
+        if constexpr (!COUPLED) {
             // decoupled form: s.xleft carries M of the cell to the left (X of the left neighbour for the lane's first
             // column -- both are valid second operands of E' = max(E + ge, .)), dd = X_diag + sigma (X form throughout)
             int x;
@@ -329,7 +333,7 @@ struct Cell {
             }
             X[C] = x;
             if constexpr (PARTIAL != 0) capture_if_bit<C>(k.capmask, s.xs, x, k.one);
-            if constexpr (C + 1 < K) Cell<LOCAL, AFFINE, K, PARTIAL, MASK, RS, RO, C + 1, TRACK, FORM>::run(X, F, sc, s, k);
+            if constexpr (C + 1 < K) Cell<LOCAL, AFFINE, K, PARTIAL, MASK, RS, RO, C + 1, COUPLED, TRACK>::run(X, F, sc, s, k);
             return;
         }
         int h;
@@ -358,7 +362,7 @@ struct Cell {
         X[C] = x;
         s.xleft = x;
         if constexpr (PARTIAL != 0) capture_if_bit<C>(k.capmask, s.xs, x, k.one);
-        if constexpr (C + 1 < K) Cell<LOCAL, AFFINE, K, PARTIAL, MASK, RS, RO, C + 1, TRACK, FORM>::run(X, F, sc, s, k);
+        if constexpr (C + 1 < K) Cell<LOCAL, AFFINE, K, PARTIAL, MASK, RS, RO, C + 1, COUPLED, TRACK>::run(X, F, sc, s, k);
     }
 };
 
@@ -379,7 +383,7 @@ struct StepStateR {
     int xs[R], es[R];    // PARTIAL: X and E of the edge column, per row
 };
 
-template <bool LOCAL, bool AFFINE, int K, int PARTIAL, bool MASK, int R, int C, int FORM = 0>
+template <bool LOCAL, bool AFFINE, int K, int PARTIAL, bool MASK, int R, int C, int FORM>
 struct CellR {
     template <int KF, int KS, int W>
     static __device__ __forceinline__ void run(int (&X)[K], int (&F)[KF], const int (&sc)[KS], StepStateR<R, W>& s,
@@ -395,18 +399,18 @@ struct CellR {
             // FORM 2 ("mixed", Gotoh two-row tiles): even rows coupled (3 ALU-pipe ops per cell), odd rows decoupled (4) --
             // the decoupled kernel is ALU-pipe bound (94 % busy, ncu), the coupled one latency bound; half and half has
             // 12 % less ALU work than the one and a short chain in every other row unlike the other
-            const bool coupled_row = (FORM == 0) || (FORM == 2 && (r & 1) == 0);
+            const bool coupled_row = FORM == 2 && (r & 1) == 0;
             if constexpr (C + 1 < K) {
                 // diagonal term of cell (r, C+1): H(r-1, C) = the cell above this one
                 if constexpr (MASK) {
-                    if (FORM == 2 && coupled_row) s.dd[r] = diag_mask_bit_c<(C + 1) * R>(s.tm, r, above_x, k.one, k.diff_c, k.same_c);
+                    if (coupled_row) s.dd[r] = diag_mask_bit_c<(C + 1) * R>(s.tm, r, above_x, k.one, k.diff_c, k.same_c);
                     else s.dd[r] = diag_mask_bit<(C + 1) * R>(s.tm, r, above_x, k);
                 } else {
                     s.dd[r] = diag_plus_sigma(s.qc[r], sc[C + 1], above_x, k.one, k.diff_o, k.same_o);
                 }
             }
             int h, x;
-            if (FORM == 2 && AFFINE && coupled_row) {
+            if (coupled_row) {
                 s.e[r] = __viaddmax_s32(s.e[r], k.ge, s.x[r]);
                 const int f = __viaddmax_s32(above_f, k.ge, above_x);
                 h = LOCAL ? __vimax3_s32_relu(dd, s.e[r], f) : __vimax3_s32(dd, s.e[r], f);
@@ -421,7 +425,7 @@ struct CellR {
                 }
                 continue;
             }
-            if constexpr ((FORM == 1 || FORM == 2) && AFFINE) {
+            if constexpr (AFFINE) {
                 // decoupled form (see Cell): s.x[r] carries M of the cell to the left, hrow holds X (= H + go)
                 const int f = __viaddmax_s32(above_f, k.ge, above_x);
                 int mp;
@@ -439,28 +443,15 @@ struct CellR {
                     capture_if_bit<C>(k.capmask, s.es[r], s.e[r], k.one);
                 }
                 continue;
-            } else if constexpr (FORM == 1) {
+            } else {
                 const int nn = LOCAL ? __viaddmax_s32_relu(above_x, k.ge, dd) : __viaddmax_s32(above_x, k.ge, dd);
                 h = __viaddmax_s32(s.x[r], k.ge, nn);
-                x = h;
-            } else if constexpr (AFFINE) {
-                s.e[r] = __viaddmax_s32(s.e[r], k.ge, s.x[r]);
-                const int f = __viaddmax_s32(above_f, k.ge, above_x);
-                h = LOCAL ? __vimax3_s32_relu(dd, s.e[r], f) : __vimax3_s32(dd, s.e[r], f);
-                x = imad_add(h, k.one, k.go);
-                above_f = f;
-            } else {
-                const int t = max(s.x[r], above_x);
-                h = LOCAL ? __viaddmax_s32_relu(t, k.ge, dd) : __viaddmax_s32(t, k.ge, dd);
                 x = h;
             }
             hrow[r] = h;
             s.x[r] = x;
             above_x = x;
-            if constexpr (PARTIAL != 0) {
-                capture_if_bit<C>(k.capmask, s.xs[r], x, k.one);
-                if constexpr (AFFINE) capture_if_bit<C>(k.capmask, s.es[r], s.e[r], k.one);   // E of the last column: Gotoh traceback joins
-            }
+            if constexpr (PARTIAL != 0) capture_if_bit<C>(k.capmask, s.xs[r], x, k.one);
         }
         if constexpr (LOCAL) {
             if constexpr (PARTIAL) {
@@ -507,7 +498,7 @@ __device__ __forceinline__ void st_record(int4* p, int4 v)
 // don't-care values (dependencies only run left->right, so they never reach a
 // valid cell), the edge column is picked out for the output, and the local
 // maximum is masked.  R = rows per lane and step (PARTIAL items use R = 1).
-template <bool LOCAL, bool AFFINE, int K, int PARTIAL, bool MASK, int R, bool TRACK = false, int FORM_SEL = 1>
+template <bool LOCAL, bool AFFINE, int K, int PARTIAL, bool MASK, int R, bool TRACK, int FORM>
 __device__ __forceinline__ bool process_item(const Job& J, const int band, const int strip,
                                              const KernelArgs& a, WarpSmem& sm,
                                              unsigned* __restrict__ s_mask /* [ncodes][32][W] spread column masks */,
@@ -520,7 +511,6 @@ __device__ __forceinline__ bool process_item(const Job& J, const int band, const
     constexpr int B = 32 / R;              // steps per batch (a batch = 32 rows)
     constexpr int QM = 64 * R - 1;         // query ring mask
     constexpr int W = TileWords<R, K>::value;
-    constexpr int FORM = TRACK ? 0 : FORM_SEL;     // the end-cell tracking kernels keep the coupled form (they need H itself)
     const int i0 = band * J.band_h;
     const int hb = min(J.band_h, J.h - i0);
     const int j0 = strip * SW;
@@ -532,11 +522,11 @@ __device__ __forceinline__ bool process_item(const Job& J, const int band, const
     k.ge = a.sp.gap_extend;
     k.go = go;
     // coupled form: dd = H_diag + sigma = X_diag + (sigma - go); decoupled form: dd = X_diag + sigma
-    k.diff_o = FORM >= 1 ? a.sp.diff : a.sp.diff - go;
-    k.same_o = FORM >= 1 ? a.sp.same : a.sp.same - go;
+    k.diff_o = TRACK ? a.sp.diff - go : a.sp.diff;
+    k.same_o = TRACK ? a.sp.same - go : a.sp.same;
     k.diff_c = a.sp.diff - go;
     k.same_c = a.sp.same - go;
-    static_assert(FORM != 2 || (MASK && AFFINE && R == 2), "mixed cells: Gotoh two-row MASK tiles");
+    static_assert(FORM == 1 || (FORM == 2 && MASK && AFFINE && R == 2), "decoupled cells, or mixed cells: Gotoh two-row MASK tiles");
     int* const status = a.status;
     const unsigned long long timeout_ns = a.timeout_ns;
 
@@ -679,7 +669,7 @@ __device__ __forceinline__ bool process_item(const Job& J, const int band, const
         dcarry = xl;
         st.xleft = xl;
         st.e = el;
-        Cell<LOCAL, AFFINE, K, PARTIAL, MASK, R, RO, 0, TRACK, (FORM == 2 ? 1 : FORM)>::run(X, F, sc, st, k);
+        Cell<LOCAL, AFFINE, K, PARTIAL, MASK, R, RO, 0, TRACK, TRACK>::run(X, F, sc, st, k);     // coupled iff tracking
         hro = st.xleft;
         ero = st.e;
         if constexpr (PARTIAL != 0) {
@@ -889,7 +879,7 @@ __device__ __forceinline__ bool process_item(const Job& J, const int band, const
         if constexpr (!PARTIAL) best = max(best, st.hprev);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(kFull, best, o));
-        if constexpr (FORM >= 1 && AFFINE) {
+        if constexpr (!TRACK && AFFINE) {
             if (best > kScoreMin) best -= go;             // the decoupled (and mixed) Gotoh cells track X = H + go
         }
         if (lane == 0) atomicMax(J.best, best);
@@ -1019,7 +1009,7 @@ strip_kernel(const KernelArgs a)
 
 using StripKernelFn = void (*)(const KernelArgs);
 // defined in strip_inst_*.cu (one translation unit per (LOCAL, AFFINE) pair)
-// form: 0 = coupled, 1 = decoupled cells; the coupled form exists for the Gotoh MASK kernels only
+// form: 1 = decoupled cells, 2 = mixed cells (Gotoh MASK kernels with K = 16 / 32 only)
 StripKernelFn get_strip_kernel_00(int K, bool mask, int form);
 StripKernelFn get_strip_kernel_01(int K, bool mask, int form);
 StripKernelFn get_strip_kernel_10(int K, bool mask, int form);

@@ -119,8 +119,8 @@ int anyseq_ctx_tune(anyseq_ctx* ctx, int cols_per_lane, int band_rows, int block
 
 /* Named options: "cols_per_lane", "band_rows", "blocks_per_sm" (warps per scheduler of the strip kernels, 1-3),
  * "watchdog_ms" (> 0), "band_slack" (band height = slack * lag * resident warps when a launch has more strips than
- * warps; default 2), "cell_form" (-1 = per launch, 0 = coupled, 1 = decoupled, 2 = mixed Gotoh cells: identical
- * results, different instruction mixes -- see DESIGN.md 3.1),
+ * warps; default 2), "cell_form" (-1 = per launch, 1 = decoupled, 2 = mixed Gotoh cells: identical results,
+ * different instruction mixes -- see DESIGN.md 3.1; other values are refused),
  * "force_generic" (1: byte-register kernels even for small alphabets), "force_affine" (1: the score path runs the
  * Gotoh kernels even for gap_init == 0 -- must equal the linear kernels; testing),
  * "align_with_score" (0: anyseq_align skips the extra score pass),
@@ -352,7 +352,7 @@ int anyseq_device_info(anyseq_ctx* ctx, int* sm_count, int* resident_warps, char
 typedef struct anyseq_launch_plan {
     int32_t cols_per_lane;        /* K: a strip is 32 * K subject columns wide */
     int32_t rows_per_step;        /* R: query rows a lane relaxes per anti-diagonal step */
-    int32_t cell_form;            /* 0 coupled, 1 decoupled, 2 mixed (DESIGN.md 3.1) */
+    int32_t cell_form;            /* 1 decoupled, 2 mixed (DESIGN.md 3.1) */
     int32_t strips;
     int32_t warps_per_scheduler;  /* 1..3: resident warps = 4 * this * sm_count */
     int32_t bands;                /* row bands; 1 when every strip has a warp of its own */

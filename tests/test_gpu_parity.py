@@ -1025,13 +1025,16 @@ def test_full_size_c3_affine_traceback_against_cpu(aligner):
     assert hashlib.sha256(np.asarray(aligner.last_split_types(), dtype=np.int32).tobytes()).hexdigest()[:16] == gold["types_sha"]
 
 
-@pytest.mark.parametrize("form", [0, 1, 2])
+@pytest.mark.parametrize("form", [1, 2])
 @pytest.mark.parametrize("K", [8, 16, 32])
 def test_both_cell_forms_vs_oracle(aligner, oracle, form, K):
-    """the coupled (round 1) and the decoupled cell form of the Gotoh kernels (strip_kernel.cuh: FORM) must both
-    reproduce the restated reference on every scheme: the engine picks a form per launch, this forces each one,
-    with several bands, 1 - 3 warps per scheduler and ragged widths"""
+    """the decoupled and the mixed cell form of the Gotoh kernels (strip_kernel.cuh: FORM) must both reproduce the
+    restated reference on every scheme: the engine picks a form per launch, this forces each one, with several
+    bands, 1 - 3 warps per scheduler and ragged widths"""
     import anyseq_b200 as A
+    with pytest.raises(A.AnyseqError) as e:           # the coupled cells (0) are not built for these kernels
+        aligner.set_option("cell_form", 0)
+    assert e.value.code == -2                          # ANYSEQ_ERR_BAD_ARG
     rng = np.random.default_rng(555 + K)
     schemes = [A.affine_scoring_scheme(2, -1, -2, -1), A.affine_scoring_scheme(5, -4, -10, -1), A.affine_scoring_scheme(1, -1, -1, 0)]
     shapes = [(300, 1025), (2100, 32 * K * 3 + 17), (1500, 32 * K * 7), (4099, 2000)]
