@@ -242,7 +242,9 @@ int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool a
     while (32 * K < ncols) K *= 2;
     // Packed 16-bit kernels (batch_x2.cu, two pairs per warp): only when every value a pair of these lengths can
     // produce fits a non-negative 16-bit half after adding `bias` (see batch_x2.cu).  Bounds: any cell is at least
-    // the all-gap path 2 gi + (rows + cols + 2) ge, at most same * min(rows, cols); columns are padded to 32 K.
+    // the all-gap path 2 gi + (rows + cols + 2) ge; at most max(same, diff, 0) * min(rows, cols), since a path has
+    // at most min(rows, cols) diagonal steps and its gap steps are <= 0 (diff > same: a run of mismatches is the
+    // best path); columns are padded to 32 K.
     int bias = 0;
     bool packed = false;
     if (use_mask_ && tune.batch_packed) {
@@ -251,7 +253,7 @@ int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool a
         const long long go = affine ? sp.gap_open : 0;
         const long long hmin = 2LL * sc.gap_init + (rows_max + cols_pad + 2) * sc.gap_extend;
         const long long lowest = hmin + go + std::min<long long>(0, std::min(sc.same, sc.diff));
-        const long long hmax = std::max<long long>(sc.same, 0) * std::min(rows_max, cols_pad);
+        const long long hmax = std::max<long long>({sc.same, sc.diff, 0}) * std::min(rows_max, cols_pad);
         const long long b = -lowest + 8;
         const long long small = std::max<long long>({std::llabs(sc.same), std::llabs(sc.diff), std::llabs(go), std::llabs(sc.gap_extend)});
         if (b + hmax + 2 * small < 32000 && small < 2000) { packed = true; bias = (int)b; }

@@ -200,7 +200,9 @@ int64_t anyseq_cigar(const char* alQuery, const char* alSubject, int64_t len, ch
 
 /* Batch of independent pairs (score only).  Sequences are packed back to back;
  * pair p is queries[q_off[p] .. q_off[p+1]) vs subjects[s_off[p] .. s_off[p+1]).
- * Host buffers; scores[npairs] is written. */
+ * Host buffers; scores[npairs] is written.  Every scheme the single-pair calls take is scored exactly, except
+ * local alignment with diff > 0: ANYSEQ_ERR_UNSUPPORTED (the kernels pad columns, and padding must not outscore
+ * real symbols).  The same holds for the packed and streaming batch entries below. */
 int anyseq_score_batch(anyseq_ctx* ctx, const anyseq_scoring* sc,
                        const char* queries, const int64_t* q_off,
                        const char* subjects, const int64_t* s_off,
