@@ -296,8 +296,7 @@ def plan_launch(mode, lenq: int, lens: int, affine: bool = False, sm_count: int 
     if scheme is None:
         rc = L.anyseq_plan_launch(int(sm_count), m, int(bool(affine)), int(lenq), int(lens), int(bool(chained)), C.byref(plan))
     else:
-        same, diff, gap_init, gap_extend = (int(v) for v in scheme)
-        sc = capi.Scoring(m, same, diff, gap_init, gap_extend)
+        sc = make_scoring(m, *scheme)
         rc = L.anyseq_plan_launch_scheme(int(sm_count), C.byref(sc), int(lenq), int(lens), int(bool(chained)), C.byref(plan))
     if rc != 0:
         raise AnyseqError(rc, L.anyseq_last_error().decode())

@@ -216,5 +216,10 @@ def _ptr(a: np.ndarray):
 
 
 def make_scoring(mode, same=2, diff=-1, gap_init=0, gap_extend=-1) -> Scoring:
+    """the C struct of a scheme; ctypes would silently wrap values outside int32 (2**32 + 5 stored as 5)"""
     m = MODES[mode] if isinstance(mode, str) else int(mode)
-    return Scoring(m, same, diff, gap_init, gap_extend)
+    vals = [int(v) for v in (same, diff, gap_init, gap_extend)]
+    for name, v in zip(("same", "diff", "gap_init", "gap_extend"), vals):
+        if not -2**31 <= v < 2**31:
+            raise ValueError(f"scoring scheme: {name} = {v} is outside int32")
+    return Scoring(m, *vals)

@@ -229,6 +229,9 @@ int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool a
                          int max_short, cudaStream_t st)
 {
     const long long npairs = ba.npairs;
+    // the bound is symmetric in the lengths and grows with both: the longest pair lengths bound every pair
+    const int rc = check_score_range(sc, max_long, max_short);
+    if (rc) return rc;
     const int limit = use_mask_ ? 1024 : 512;
     int cols_longer, ncols;
     if (max_long <= limit) { cols_longer = 1; ncols = max_long; }

@@ -256,6 +256,8 @@ int Engine::align_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, con
     bool negative;
     if ((rc = batch_len_stats(ba, &max_long, &max_short, &max_q, &max_s, &negative))) return rc;
     if (negative) { set_last_error("batch offsets must be non-decreasing"); return ANYSEQ_ERR_BAD_ARG; }
+    // the bound grows with both lengths: the longest query and subject bound every pair
+    if ((rc = check_score_range(sc, max_q, max_s))) return rc;
     if (max_s > kMaxAlignBatchSubject) {
         char buf[200];
         std::snprintf(buf, sizeof(buf), "batch traceback: a subject of %d symbols is longer than %d; "

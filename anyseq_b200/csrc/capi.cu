@@ -363,9 +363,11 @@ int anyseq_plan_launch_scheme(int sm_count, const anyseq_scoring* sc, int lenq, 
     anyseq::ScoreParams sp;
     bool affine = false;
     if (!sc) return ANYSEQ_ERR_BAD_ARG;
-    const int rc = anyseq::make_score_params(*sc, &sp, &affine);
+    int rc = anyseq::make_score_params(*sc, &sp, &affine);
     if (rc) return rc;
-    anyseq::Engine planner;           // never init()ed: no device, no buffers -- only the planning members are used
+    // the launch would be refused: so is its plan (a device-free way to ask whether a problem is in range)
+    if ((rc = anyseq::check_score_range(*sc, lenq, lens))) return rc;
+    anyseq::Engine planner;          // never init()ed: no device, no buffers -- only the planning members are used
     return planner.plan_launch(sm_count, sc->mode, affine, lenq, lens, chained != 0, sp, out);
 }
 

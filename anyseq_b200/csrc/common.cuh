@@ -9,7 +9,7 @@ namespace anyseq {
 
 constexpr int kWarp = 32;
 // "minus infinity" for the affine E/F borders (SURVEY.md A.7: MIN/2 so that
-// adding gap costs cannot wrap).  Scores must stay inside (-2^29, 2^29).
+// adding gap costs cannot wrap).  check_score_range (engine.cu) refuses problems whose scores come near it or INT_MAX.
 constexpr int kNegInf = -(1 << 30);
 // reference SCORE_MIN_VALUE: src/align.impala:16
 constexpr int kScoreMin = -2147483647;

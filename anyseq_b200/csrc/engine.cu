@@ -699,12 +699,44 @@ int Engine::run_jobs(std::vector<Job>& jobs, const ScoreParams& sp, bool local, 
     return ANYSEQ_OK;
 }
 
+// Cells are 32-bit with minus infinity kNegInf = -2^30.  lo and hi bound every H of an m x n problem: hi is the score
+// of a path with min(m, n) diagonal steps of the best symbol score, lo the larger of an all-gap path and a diagonal-then-
+// gap path (global), of the diagonal from the border and a single gap from the border (semiglobal), or 0 (local).  E
+// and F stay within [lo + go, hi].  The 4 P margin covers the few additions a cell makes (+ sigma, + go, + ge, the
+// decoupled X = H + go), so kNegInf + ge stays below every real candidate and no sum wraps.  Padded cells only feed
+// padded cells, so the real lengths decide.  The Hirschberg joins add two halves of one alignment through the split
+// (plus -gi for an E join), which the whole problem's bound covers.
+int check_score_range(const anyseq_scoring& sc, long long m, long long n)
+{
+    const long long same = sc.same, diff = sc.diff, gi = sc.gap_init, ge = sc.gap_extend;
+    const long long P = std::max({std::llabs(same), std::llabs(diff), std::llabs(gi), std::llabs(ge)});
+    bool ok = P <= (1LL << 24);
+    if (ok) {                         // P <= 2^24 and lengths < 2^31: every product below fits 64 bits
+        const long long k = std::min(m, n), sigma = std::min({0LL, same, diff});
+        const long long hi = std::max({same, diff, 0LL}) * k;
+        long long lo = 0;
+        if (sc.mode == ANYSEQ_GLOBAL) lo = std::max(2 * gi + (m + n) * ge, sigma * k + gi + (std::max(m, n) - 1) * ge);
+        else if (sc.mode == ANYSEQ_SEMIGLOBAL) lo = std::max(sigma * k, gi + k * ge);
+        ok = hi <= 0x7fffffffLL - 4 * P && lo >= (long long)kNegInf + 4 * P;
+    }
+    if (ok) return ANYSEQ_OK;
+    char buf[256];
+    std::snprintf(buf, sizeof(buf), "scores of a %lld x %lld problem under (%d, %d, %d, %d) leave the 32-bit cell range: "
+                  "|same|, |diff|, |gap_init|, |gap_extend| <= 2^24 and every score within [-2^30 + 4 P, 2^31 - 1 - 4 P] "
+                  "(P = the largest of them)", m, n, sc.same, sc.diff, sc.gap_init, sc.gap_extend);
+    set_last_error(buf);
+    return ANYSEQ_ERR_UNSUPPORTED;
+}
+
 int make_score_params(const anyseq_scoring& sc, ScoreParams* sp, bool* affine)
 {
     if (sc.mode < 0 || sc.mode > 2 || sc.gap_init > 0 || sc.gap_extend > 0) {
         set_last_error("bad scoring scheme (mode in 0..2, gap costs must be <= 0)");
         return ANYSEQ_ERR_BAD_ARG;
     }
+    // an empty problem: only the magnitude limit of the cell range applies (gap_init + gap_extend must not wrap)
+    const int rc = check_score_range(sc, 0, 0);
+    if (rc) return rc;
     *affine = sc.gap_init != 0;
     sp->same = sc.same;
     sp->diff = sc.diff;
@@ -761,6 +793,8 @@ int Engine::score_strip_device(const anyseq_scoring& sc, const uint8_t* d_q, int
     affine = affine || tune.force_affine;
     const int w = col_end - col_begin;
     if (m < 1 || w < 1 || col_begin < 0 || col_end > n_total) { set_last_error("bad strip range"); return ANYSEQ_ERR_BAD_ARG; }
+    // the whole problem, not the slice: a rank's narrow slice of an out-of-range problem is out of range too
+    if ((rc = check_score_range(sc, m, n_total))) return rc;
     // the strips read / write one border record per query row of the inboxes (the next rank's lives in PEER memory)
     if ((inbox && m > inbox->rows) || (next_inbox && m > next_inbox->rows)) {
         set_last_error("query longer than the rows the inbox was created with");
@@ -912,6 +946,7 @@ int Engine::score_strip_device_multi(const anyseq_scoring& sc, int npairs, const
     affine = affine || tune.force_affine;
     const int w = col_end - col_begin;
     if (m < 1 || w < 1 || col_begin < 0 || col_end > n_total) { set_last_error("bad strip range"); return ANYSEQ_ERR_BAD_ARG; }
+    if ((rc = check_score_range(sc, m, n_total))) return rc;
     for (int p = 0; p < npairs; ++p) {
         if ((inbox && inbox[p] && m > inbox[p]->rows) || (next_inbox && next_inbox[p] && m > next_inbox[p]->rows)) {
             set_last_error("query longer than the rows the inbox was created with");

@@ -210,6 +210,9 @@ private:
 };
 
 void set_last_error(const std::string& s);
+// engine.cu: ANYSEQ_ERR_UNSUPPORTED when some score of an m x n problem under sc may leave the 32-bit cell range
+// (include/anyseq.h states the rule); every entry point that launches DP kernels calls it with the real lengths
+int check_score_range(const anyseq_scoring& sc, long long m, long long n);
 int make_score_params(const anyseq_scoring& sc, ScoreParams* sp, bool* affine);
 // batch.cu: the checks every batch entry point starts with -- the scheme, a cleared *out, and local alignment with
 // diff > 0 refused for a non-empty batch (padded columns must not outscore real ones)

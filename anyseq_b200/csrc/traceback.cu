@@ -294,6 +294,7 @@ int Engine::align_host(const anyseq_scoring& sc, const char* q, int m, const cha
         out->score = tmp.score;
         return ANYSEQ_OK;
     }
+    if ((rc = check_score_range(sc, m, n))) return rc;
 
     const bool local = sc.mode == ANYSEQ_LOCAL;
     const int glob = sc.mode == ANYSEQ_GLOBAL;

@@ -124,6 +124,7 @@ int Engine::align_full_host(const anyseq_scoring& sc, const char* q, int m, cons
     std::memset(als, ' ', total);
     if (start2) start2[0] = start2[1] = 0;
     if (m == 0 || n == 0) return score_host(sc, q, m, s, n, out);     // nothing to relax: degenerate result, blank rows
+    if ((rc = check_score_range(sc, m, n))) return rc;
     std::lock_guard<std::recursive_mutex> lock(mu_);
     ANYSEQ_CUDA_CHECK(cudaSetDevice(device));
 

@@ -89,7 +89,18 @@ enum {                       /* status codes (0 = ok, < 0 = failure) */
  * gap_init < 0 selects Gotoh affine gaps: a gap of length L costs
  * gap_init + L*gap_extend (parameter names of affine_scoring_scheme,
  * src/align.impala:153-154; the recurrence itself is defined by this build,
- * see DESIGN.md -- the reference only ships an uncalled stub). */
+ * see DESIGN.md -- the reference only ships an uncalled stub).
+ *
+ * Score range: cells are 32-bit with minus infinity -2^30, so every call that runs DP kernels refuses, with
+ * ANYSEQ_ERR_UNSUPPORTED, a problem whose scores could leave that range; every problem it accepts is scored exactly.
+ * With P = max(|same|, |diff|, |gap_init|, |gap_extend|), k = min(m, n) and sigma = min(0, same, diff), an m x n
+ * problem (batches: the longest query and subject; multi-GPU slices: the whole problem) is accepted iff
+ *   P <= 2^24,  max(same, diff, 0) * k <= 2^31 - 1 - 4 P  and  lo >= -2^30 + 4 P, where lo is
+ *   global:     max(2 gap_init + (m + n) gap_extend,  sigma k + gap_init + (max(m, n) - 1) gap_extend)
+ *   semiglobal: max(sigma k,  gap_init + k gap_extend)
+ *   local:      0
+ * E.g. a 4.6 Mbp pair takes same <= 466 semiglobally and locally.  anyseq_plan_launch_scheme applies the same rule
+ * without a device. */
 typedef struct anyseq_scoring {
     int32_t mode;            /* ANYSEQ_GLOBAL / SEMIGLOBAL / LOCAL */
     int32_t same;            /* score of equal symbols (bytes compared raw) */
