@@ -223,6 +223,36 @@ class Aligner:
                                                         C.byref(res)))
         return AlignmentResult(res.score, -1, -1, res.kernel_ms, res.kernel_launches)
 
+    def score_batch_ends(self, mode, queries, q_off, subjects, s_off, scoring: ScoringScheme = REFERENCE_SCORING):
+        """score_batch plus the end cell of every pair: -> (scores, ends (npairs, 2) int32 of (end_i, end_j),
+        AlignmentResult).  The end cells are those score() reports for each pair alone (local alignment: with the
+        option "local_end_cell" set); local batches need subjects of at most 1024 symbols (512 for large alphabets)."""
+        q, s = as_u8(queries), as_u8(subjects)
+        qo = np.ascontiguousarray(q_off, dtype=np.int64)
+        so = np.ascontiguousarray(s_off, dtype=np.int64)
+        npairs = len(qo) - 1
+        scores = np.zeros(max(npairs, 1), dtype=np.int32)
+        ends = np.zeros((max(npairs, 1), 2), dtype=np.int32)
+        sc = make_scoring(mode, scoring.same, scoring.diff, scoring.gap_init, scoring.gap_extend)
+        res = Result()
+        i64p, i32p = C.POINTER(C.c_int64), C.POINTER(C.c_int32)
+        self._check(self._lib.anyseq_score_batch_ends(self._ctx, C.byref(sc), capi._ptr(q), qo.ctypes.data_as(i64p),
+                                                      capi._ptr(s), so.ctypes.data_as(i64p), npairs,
+                                                      scores.ctypes.data_as(i32p), ends.ctypes.data_as(i32p),
+                                                      C.byref(res)))
+        return scores[:npairs], ends[:npairs], AlignmentResult(res.score, -1, -1, res.kernel_ms, res.kernel_launches)
+
+    def score_batch_ends_device(self, mode, d_queries: int, d_q_off: int, d_subjects: int, d_s_off: int, npairs: int,
+                                d_scores: int, d_ends: int, scoring: ScoringScheme = REFERENCE_SCORING) -> AlignmentResult:
+        """score_batch_ends on device memory (raw pointers); d_ends holds 2 * npairs int32"""
+        sc = make_scoring(mode, scoring.same, scoring.diff, scoring.gap_init, scoring.gap_extend)
+        res = Result()
+        vp = C.c_void_p
+        self._check(self._lib.anyseq_score_batch_ends_device(self._ctx, C.byref(sc), vp(d_queries), vp(d_q_off),
+                                                             vp(d_subjects), vp(d_s_off), npairs, vp(d_scores),
+                                                             vp(d_ends or None), C.byref(res)))
+        return AlignmentResult(res.score, -1, -1, res.kernel_ms, res.kernel_launches)
+
     # -- full-matrix tracebacks of batches (anyseq_align_batch) --------------
     def align_batch(self, mode, queries, q_off, subjects, s_off, scoring: ScoringScheme = REFERENCE_SCORING) -> BatchAlignment:
         """traceback_full of every pair (as align_full) in one launch; every subject <= 1024 symbols"""
@@ -263,19 +293,26 @@ class Aligner:
 
     # -- 2-bit packed DNA batches (anyseq_score_batch_packed2) -----------------
     def score_batch_packed2(self, mode, batch: "capi.PackedBatch", scores, scoring: ScoringScheme = REFERENCE_SCORING,
-                            device: bool = False) -> AlignmentResult:
+                            device: bool = False, ends=None) -> AlignmentResult:
         """batch: capi.PackedBatch with host addresses (device=False: chunks are copied from the caller's memory under
         the kernels; pin the arrays for full H2D speed) or device addresses (device=True); scores: address of npairs
-        int32 (host resp. device)"""
+        int32 (host resp. device); ends: optional address of 2 * npairs int32 for the end cells (see score_batch_ends)"""
         sc = make_scoring(mode, scoring.same, scoring.diff, scoring.gap_init, scoring.gap_extend)
         res = Result()
-        fn = self._lib.anyseq_score_batch_packed2_device if device else self._lib.anyseq_score_batch_packed2
-        self._check(fn(self._ctx, C.byref(sc), C.byref(batch), C.c_void_p(int(scores)), C.byref(res)))
+        if ends is None:
+            fn = self._lib.anyseq_score_batch_packed2_device if device else self._lib.anyseq_score_batch_packed2
+            self._check(fn(self._ctx, C.byref(sc), C.byref(batch), C.c_void_p(int(scores)), C.byref(res)))
+        else:
+            fn = self._lib.anyseq_score_batch_packed2_ends_device if device else self._lib.anyseq_score_batch_packed2_ends
+            self._check(fn(self._ctx, C.byref(sc), C.byref(batch), C.c_void_p(int(scores)), C.c_void_p(int(ends) or None),
+                           C.byref(res)))
         return AlignmentResult(res.score, -1, -1, res.kernel_ms, res.kernel_launches)
 
     def batch_stream(self, mode, scoring: ScoringScheme = REFERENCE_SCORING, cap_pairs: int = 1 << 17,
-                     cap_query_bytes: int = 32 << 20, cap_subject_bytes: int = 32 << 20, slots: int = 3) -> "BatchStream":
-        return BatchStream(self, mode, scoring, cap_pairs, cap_query_bytes, cap_subject_bytes, slots)
+                     cap_query_bytes: int = 32 << 20, cap_subject_bytes: int = 32 << 20, slots: int = 3,
+                     ends: bool = False) -> "BatchStream":
+        """ends=True: every collected chunk also carries the end cells of its pairs (BatchStream.chunk_ends)"""
+        return BatchStream(self, mode, scoring, cap_pairs, cap_query_bytes, cap_subject_bytes, slots, ends)
 
     # -- roofline denominator ----------------------------------------------
     def measure_int_peak(self, kind: int = 0):
@@ -331,12 +368,13 @@ class BatchStream:
     are pinned host memory owned by the stream, exposed as numpy views."""
 
     def __init__(self, aligner: Aligner, mode, scoring: ScoringScheme, cap_pairs: int, cap_query_bytes: int,
-                 cap_subject_bytes: int, slots: int = 3):
+                 cap_subject_bytes: int, slots: int = 3, ends: bool = False):
         self._al, self._lib = aligner, aligner._lib
         sc = make_scoring(mode, scoring.same, scoring.diff, scoring.gap_init, scoring.gap_extend)
         self._h = C.c_void_p()
-        aligner._check(self._lib.anyseq_batch_stream_open(aligner.handle, C.byref(sc), cap_pairs, cap_query_bytes,
-                                                          cap_subject_bytes, slots, C.byref(self._h)))
+        fn = self._lib.anyseq_batch_stream_open_ends if ends else self._lib.anyseq_batch_stream_open
+        aligner._check(fn(aligner.handle, C.byref(sc), cap_pairs, cap_query_bytes, cap_subject_bytes, slots,
+                          C.byref(self._h)))
 
     @staticmethod
     def _view(addr, n, dtype):
@@ -369,6 +407,14 @@ class BatchStream:
             return None
         self._al._check(rc)
         return c, self._view(C.cast(c.scores, C.c_void_p).value, c.npairs, np.int32)
+
+    def chunk_ends(self, chunk):
+        """end cells of a collected chunk: (npairs, 2) int32 view valid until release; None for a stream opened
+        without ends"""
+        p = self._lib.anyseq_batch_stream_chunk_ends(self._h, C.byref(chunk))
+        if not p:
+            return None
+        return self._view(C.cast(p, C.c_void_p).value, 2 * chunk.npairs, np.int32).reshape(-1, 2)
 
     def release(self, chunk):
         self._al._check(self._lib.anyseq_batch_stream_release(self._h, C.byref(chunk)))

@@ -20,7 +20,7 @@ LIB_SOURCES = ["engine.cu", "capi.cu", "microbench.cu", "inbox.cu", "traceback.c
                "strip_inst_00.cu", "strip_inst_01.cu", "strip_inst_10.cu", "strip_inst_11.cu",
                "strip_inst_10t.cu", "strip_inst_11t.cu", "strip_inst_01p.cu"]
 CLI_SOURCES = ["align_main.cpp", "sequence_io.cpp", "alignment_io.cpp"]
-HEADERS = ["common.cuh", "engine.cuh", "strip_kernel.cuh", "strip_packed.cuh", "strip_inst.inl", "batch.cuh", "traceback_full.cuh", "sequence_io.h", "alignment_io.h",
+HEADERS = ["common.cuh", "engine.cuh", "strip_kernel.cuh", "strip_packed.cuh", "strip_inst.inl", "batch.cuh", "batch_kernel_body.inl", "traceback_full.cuh", "sequence_io.h", "alignment_io.h",
            os.path.join("..", "..", "include", "anyseq.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -26,9 +26,11 @@ EXPORTED_SYMBOLS = [
     "anyseq_align_full", "anyseq_align_sharded", "anyseq_align_batch", "anyseq_align_batch_device",
     "anyseq_ctx_create", "anyseq_ctx_destroy", "anyseq_last_error", "anyseq_ctx_tune", "anyseq_ctx_set_option",
     "anyseq_score", "anyseq_score_device", "anyseq_align", "anyseq_last_splits", "anyseq_last_split_types", "anyseq_cigar",
-    "anyseq_score_batch", "anyseq_score_batch_device",
+    "anyseq_score_batch", "anyseq_score_batch_device", "anyseq_score_batch_ends", "anyseq_score_batch_ends_device",
     "anyseq_score_batch_packed2", "anyseq_score_batch_packed2_device", "anyseq_pack2",
-    "anyseq_batch_stream_open", "anyseq_batch_stream_acquire", "anyseq_batch_stream_submit", "anyseq_batch_stream_finish",
+    "anyseq_score_batch_packed2_ends", "anyseq_score_batch_packed2_ends_device",
+    "anyseq_batch_stream_open", "anyseq_batch_stream_open_ends", "anyseq_batch_stream_chunk_ends",
+    "anyseq_batch_stream_acquire", "anyseq_batch_stream_submit", "anyseq_batch_stream_finish",
     "anyseq_batch_stream_collect", "anyseq_batch_stream_release", "anyseq_batch_stream_stats", "anyseq_batch_stream_close",
     "anyseq_strip_inbox_create", "anyseq_strip_inbox_open", "anyseq_strip_inbox_reset",
     "anyseq_strip_inbox_destroy", "anyseq_score_strip_device", "anyseq_score_strip", "anyseq_score_strip_device_multi", "anyseq_strip_combine",
@@ -147,6 +149,17 @@ def load_library(path: str | None = None):
                                      C.POINTER(C.c_int32), C.POINTER(Result)]
     L.anyseq_score_batch_device.restype = C.c_int
     L.anyseq_score_batch_device.argtypes = [vp, C.POINTER(Scoring), vp, vp, vp, vp, C.c_int64, vp, C.POINTER(Result)]
+    L.anyseq_score_batch_ends.restype = C.c_int
+    L.anyseq_score_batch_ends.argtypes = [vp, C.POINTER(Scoring), vp, i64p, vp, i64p, C.c_int64,
+                                          C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(Result)]
+    L.anyseq_score_batch_ends_device.restype = C.c_int
+    L.anyseq_score_batch_ends_device.argtypes = [vp, C.POINTER(Scoring), vp, vp, vp, vp, C.c_int64, vp, vp,
+                                                 C.POINTER(Result)]
+    L.anyseq_score_batch_packed2_ends.restype = C.c_int
+    L.anyseq_score_batch_packed2_ends.argtypes = [vp, C.POINTER(Scoring), C.POINTER(PackedBatch), vp, vp, C.POINTER(Result)]
+    L.anyseq_score_batch_packed2_ends_device.restype = C.c_int
+    L.anyseq_score_batch_packed2_ends_device.argtypes = [vp, C.POINTER(Scoring), C.POINTER(PackedBatch), vp, vp,
+                                                         C.POINTER(Result)]
     L.anyseq_score_batch_packed2.restype = C.c_int
     L.anyseq_score_batch_packed2.argtypes = [vp, C.POINTER(Scoring), C.POINTER(PackedBatch), vp, C.POINTER(Result)]
     L.anyseq_score_batch_packed2_device.restype = C.c_int
@@ -155,6 +168,10 @@ def load_library(path: str | None = None):
     L.anyseq_pack2.argtypes = [vp, C.c_int64, vp]
     L.anyseq_batch_stream_open.restype = C.c_int
     L.anyseq_batch_stream_open.argtypes = [vp, C.POINTER(Scoring), C.c_int64, C.c_int64, C.c_int64, C.c_int, C.POINTER(vp)]
+    L.anyseq_batch_stream_open_ends.restype = C.c_int
+    L.anyseq_batch_stream_open_ends.argtypes = [vp, C.POINTER(Scoring), C.c_int64, C.c_int64, C.c_int64, C.c_int, C.POINTER(vp)]
+    L.anyseq_batch_stream_chunk_ends.restype = C.POINTER(C.c_int32)
+    L.anyseq_batch_stream_chunk_ends.argtypes = [vp, C.POINTER(BatchChunk)]
     for name in ("acquire", "submit", "collect", "release"):
         f = getattr(L, "anyseq_batch_stream_" + name)
         f.restype = C.c_int

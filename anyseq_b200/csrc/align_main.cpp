@@ -14,7 +14,8 @@
 // Addition (SURVEY 8f.2): align (-b|--batch) <reads file> <windows file> pairs record k of the first
 // file with record k of the second and streams them through anyseq_batch_stream_*: a reader thread
 // parses FASTA/FASTQ records straight into pinned chunk buffers while the GPU scores the previous
-// chunk; one line "<index>\t<score>" per pair.  --mode/--same/--diff/--gap-init/--gap-extend pick
+// chunk; one line "<index>\t<score>" per pair (with --ends "<index>\t<score>\t<end_i>\t<end_j>": the end cell
+// anyseq_score reports for the pair, see anyseq_score_batch_ends).  --mode/--same/--diff/--gap-init/--gap-extend pick
 // the scheme (default: the reference's linear 2/-1/-1, global).
 #include <algorithm>
 #include <chrono>
@@ -90,7 +91,7 @@ std::string random_dna(std::int64_t lo, std::int64_t hi, Rng& rng)
 }
 
 // producer: records -> pinned chunk buffers; consumer: scores -> os
-int run_batch(const std::string& reads, const std::string& windows, const anyseq_scoring& sc, std::ostream& os)
+int run_batch(const std::string& reads, const std::string& windows, const anyseq_scoring& sc, bool ends, std::ostream& os)
 {
     anyseq_ctx* ctx = nullptr;
     if (anyseq_ctx_create(-1, &ctx) != ANYSEQ_OK) { std::cerr << anyseq_last_error() << std::endl; return 1; }
@@ -105,7 +106,9 @@ int run_batch(const std::string& reads, const std::string& windows, const anyseq
     }
     const std::int64_t cap_pairs = 1 << 17, cap_bytes = 48 << 20;
     anyseq_batch_stream* st = nullptr;
-    if (anyseq_batch_stream_open(ctx, &sc, cap_pairs, cap_bytes, cap_bytes, 3, &st) != ANYSEQ_OK) {
+    const int orc = ends ? anyseq_batch_stream_open_ends(ctx, &sc, cap_pairs, cap_bytes, cap_bytes, 3, &st)
+                         : anyseq_batch_stream_open(ctx, &sc, cap_pairs, cap_bytes, cap_bytes, 3, &st);
+    if (orc != ANYSEQ_OK) {
         std::cerr << anyseq_last_error() << std::endl;
         anyseq_ctx_destroy(ctx);
         return 1;
@@ -153,7 +156,13 @@ int run_batch(const std::string& reads, const std::string& windows, const anyseq
         const int r = anyseq_batch_stream_collect(st, &c);
         if (r == ANYSEQ_EOF) break;
         if (r != ANYSEQ_OK) { std::cerr << anyseq_last_error() << std::endl; rc = 1; break; }
-        for (std::int64_t k = 0; k < c.npairs; ++k) os << ++index << '\t' << c.scores[k] << '\n';
+        if (ends) {
+            const int32_t* e = anyseq_batch_stream_chunk_ends(st, &c);
+            for (std::int64_t k = 0; k < c.npairs; ++k)
+                os << ++index << '\t' << c.scores[k] << '\t' << e[2 * k] << '\t' << e[2 * k + 1] << '\n';
+        } else {
+            for (std::int64_t k = 0; k < c.npairs; ++k) os << ++index << '\t' << c.scores[k] << '\n';
+        }
         anyseq_batch_stream_release(st, &c);
     }
     if (rc) {
@@ -174,13 +183,14 @@ void usage(const char* argv0)
     std::cout << "SYNOPSIS\n"
               << "        " << argv0 << " [-o <file>] [-p] (-i|--in) <query file> <subject file>\n"
               << "        " << argv0 << " [-o <file>] [-p] (-r|--rand) [<min len>] [<max len>]\n"
-              << "        " << argv0 << " [-o <file>] [scheme] (-b|--batch) <reads file> <windows file>\n\n"
+              << "        " << argv0 << " [-o <file>] [scheme] [--ends] (-b|--batch) <reads file> <windows file>\n\n"
               << "OPTIONS\n"
               << "        -i, --in    read sequences from input files (first record of each)\n"
               << "        -r, --rand  generate random input sequences\n"
               << "        -o, --out   write results to file\n"
               << "        -p, --print print the alignments (print_alignment format)\n"
               << "        -b, --batch score record k of the first file against record k of the second\n"
+              << "        --ends      with --batch: also print the end cell (end_i, end_j) of every pair\n"
               << "        scheme:     [--mode global|semiglobal|local] [--same <n>] [--diff <n>]\n"
               << "                    [--gap-init <n>] [--gap-extend <n>]   (default: global 2 -1 0 -1)\n";
 }
@@ -203,7 +213,7 @@ int main(int argc, char* argv[])
     anyseq_scoring sc = {ANYSEQ_GLOBAL, 2, -1, 0, -1};
     std::string query, subject, outfile;
     std::int64_t minlen = 256, maxlen = 1024;     // reference defaults (src/main.cpp:134-135)
-    bool print = false, bad = false, want_out = false;
+    bool print = false, bad = false, want_out = false, ends = false;
     std::vector<std::string> unknown;
 
     for (int k = 1; k < argc; ++k) {
@@ -213,6 +223,8 @@ int main(int argc, char* argv[])
             if (k + 1 < argc) outfile = argv[++k]; else bad = true;
         } else if (a == "-p" || a == "--print") {
             print = true;
+        } else if (a == "--ends") {
+            ends = true;
         } else if ((a == "-i" || a == "--in") && input == Input::none) {
             input = Input::file;
             if (k + 2 < argc) { query = argv[++k]; subject = argv[++k]; } else bad = true;
@@ -241,6 +253,7 @@ int main(int argc, char* argv[])
             unknown.push_back(a);
         }
     }
+    if (ends && input != Input::batch) bad = true;
     if (bad || input == Input::none || !unknown.empty()) {
         if (!unknown.empty()) {
             std::cout << "Unknown command line arguments:\n";
@@ -256,9 +269,9 @@ int main(int argc, char* argv[])
             if (outfile.empty()) { std::cerr << "No output file name given!" << std::endl; return 1; }
             std::ofstream os(outfile);
             if (!os.good()) { std::cerr << "Unable to open output file!" << std::endl; return 1; }
-            return run_batch(query, subject, sc, os);
+            return run_batch(query, subject, sc, ends, os);
         }
-        return run_batch(query, subject, sc, std::cout);
+        return run_batch(query, subject, sc, ends, std::cout);
     }
 
     if (input == Input::file) {

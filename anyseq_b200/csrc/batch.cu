@@ -48,193 +48,92 @@ __global__ void batch_stats_kernel(const BatchArgs a, int* __restrict__ stats)
     }
 }
 
+// The body of batch_kernel / batch_ends_kernel, included into both so that each is a kernel of its own code (as a
+// shared inline function the body compiles to different SASS for the score-only kernels)
 template <int MODE, bool AFFINE, int K, bool MASK>
 __global__ void __launch_bounds__(kThreads, (K >= 32 ? 4 : (K >= 16 ? 5 : 6))) batch_kernel(const BatchArgs a)
 {
-    constexpr bool LOCAL = MODE == kLocal;
-    constexpr bool GLOB = MODE == kGlobal;
-    __shared__ uint8_t s_rows[kWarpsPerBlock][64];
-    __shared__ uint8_t s_lut[MASK ? 256 : 4];
-    extern __shared__ unsigned s_dyn[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if constexpr (MASK) {
-        if (!a.packed2) {
-            for (int x = threadIdx.x; x < 256; x += kThreads) s_lut[x] = a.lut[x];
-        }
-        __syncthreads();
-    }
-    unsigned* s_mask = s_dyn + warp * a.ncodes * 32;
-    uint8_t* rq = s_rows[warp];
-    rq[lane] = 0;
-    rq[32 + lane] = 0;
-    __syncwarp();
-
-    const int go = AFFINE ? a.sp.gap_open : 0;
-    StepConst k;
-    k.one = a.one;
-    k.ge = a.sp.gap_extend;
-    k.go = go;
-    k.diff_o = a.sp.diff - go;
-    k.same_o = a.sp.same - go;
-    k.nvalid = K;
-    k.outc = K - 1;
-    // border(k) = H(k,-1) = H(-1,k): src/align.impala:85-86 (+ Gotoh opening cost)
-    auto border = [&](int idx) -> int { return GLOB ? a.sp.gap_open + idx * a.sp.gap_extend : 0; };
-
-    long long pair = (long long)blockIdx.x * kWarpsPerBlock + warp;
-    while (pair < a.npairs) {
-        const long long q0 = batch_q_start(a, pair), s0 = batch_s_start(a, pair);
-        const int lq = batch_q_len(a, pair), ls = batch_s_len(a, pair);
-        int score;
-        if (lq == 0 || ls == 0) {
-            score = empty_pair_score<MODE>(a, lq, ls);
-        } else {
-            const bool q_is_cols = a.cols_longer ? (lq >= ls) : (lq < ls);
-            const uint8_t* cols = q_is_cols ? a.q + q0 : a.s + s0;
-            const uint8_t* rows = q_is_cols ? a.s + s0 : a.q + q0;
-            const int n = q_is_cols ? lq : ls;      // columns (<= 32*K)
-            const int m = q_is_cols ? ls : lq;      // rows
-
-            int X[K], F[AFFINE ? K : 1], sc[MASK ? 1 : K];
-            const int jl = lane * K;
-#pragma unroll
-            for (int c = 0; c < K; ++c) X[c] = border(jl + c) + go;
-            if constexpr (AFFINE) {
-#pragma unroll
-                for (int c = 0; c < K; ++c) F[c] = kNegInf;
-            } else {
-                F[0] = 0;
-            }
-            if constexpr (MASK) {
-                sc[0] = 0;
-                __syncwarp();
-                for (int cd = 0; cd < a.ncodes; ++cd) s_mask[cd * 32 + lane] = 0u;
-#pragma unroll 4
-                for (int c = 0; c < K; ++c) {
-                    const int j = jl + c;
-                    const int cd = (j < n) ? batch_code(cols, j, a.packed2, s_lut) : 0;
-                    if (cd) s_mask[cd * 32 + lane] |= 1u << c;
-                }
-                __syncwarp();
-            } else {
-#pragma unroll
-                for (int c = 0; c < K; ++c) sc[c] = (jl + c < n) ? (int)cols[jl + c] : 0x7fff;
-            }
-            int dcarry = (lane == 0) ? go : border(jl - 1) + go;     // H(-1, jl-1) in X form; H(-1,-1) = 0
-            const int outlane = (n - 1) / K, outc = (n - 1) % K;
-            int hr = 0, er = 0;
-            int colbest = kScoreMin;     // semiglobal: max over H(i, n-1), kept by lane `outlane`
-            StepState<1> st;
-            st.dd = 0; st.e = 0; st.xleft = 0; st.best = kScoreMin; st.hprev = kScoreMin; st.es = 0; st.xs = 0; st.tm[0] = 0u; st.qc = 0;
-            auto row_mask = [&](int i) -> unsigned { return s_mask[(int)rq[i & 63] * 32 + lane]; };
-            const int T = m + outlane;
-            for (int tb = 0; tb < T; tb += 32) {
-                __syncwarp();
-                {
-                    const int r = tb + lane;
-                    uint8_t v = 0;
-                    if (r < m) v = MASK ? (uint8_t)batch_code(rows, r, a.packed2, s_lut) : rows[r];
-                    rq[r & 63] = v;
-                    __syncwarp();
-                    if constexpr (MASK) st.tm[0] = row_mask(tb - lane);
-                }
-                const int tend = min(tb + 32, T);
-#pragma unroll 1
-                for (int t = tb; t < tend; ++t) {
-                    int xl = __shfl_up_sync(kFull, hr, 1);
-                    int el = 0;
-                    if constexpr (AFFINE) el = __shfl_up_sync(kFull, er, 1);
-                    const int i = t - lane;
-                    if (lane == 0) { xl = border(i) + go; el = kNegInf; }
-                    unsigned mask_next = 0u;
-                    if constexpr (MASK) mask_next = row_mask(i + 1);
-                    if ((unsigned)i < (unsigned)m) {
-                        if constexpr (MASK) {
-                            st.dd = diag_plus_sigma_mask<0>(st.tm[0], dcarry, k.one, k.diff_o, k.same_o);
-                        } else {
-                            st.qc = rq[i & 63];
-                            st.dd = diag_plus_sigma(st.qc, sc[0], dcarry, k.one, k.diff_o, k.same_o);
-                        }
-                        dcarry = xl;
-                        st.xleft = xl;
-                        st.e = el;
-                        Cell<LOCAL, AFFINE, K, false, MASK, 1, 0, 0, true>::run(X, F, sc, st, k);    // coupled cells
-                        hr = st.xleft;
-                        er = st.e;
-                        if constexpr (MODE == kSemiglobal) {
-                            if (lane == outlane) colbest = max(colbest, pick_column(X, outc));
-                        }
-                    }
-                    if constexpr (MASK) st.tm[0] = mask_next;
-                }
-            }
-            // result extraction: src/scoring.impala:29-137 (values only)
-            if constexpr (GLOB) {
-                score = __shfl_sync(kFull, pick_column(X, outc), outlane) - go;
-            } else if constexpr (MODE == kSemiglobal) {
-                int best = colbest;
-#pragma unroll
-                for (int c = 0; c < K; ++c)
-                    if (jl + c < n) best = max(best, X[c]);           // last row H(m-1, j)
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(kFull, best, o));
-                score = max(best - go, 0);                             // candidates H(m-1,-1) = H(-1,n-1) = 0
-            } else {
-                int best = st.best;
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) best = max(best, __shfl_xor_sync(kFull, best, o));
-                score = best;
-            }
-        }
-        if (lane == 0) a.scores[pair] = score;
-        unsigned long long nxt = 0;
-        if (lane == 0) nxt = atomicAdd(a.counter, 1ull);
-        pair = (long long)__shfl_sync(kFull, nxt, 0);
-    }
+    constexpr bool ENDS = false;
+#include "batch_kernel_body.inl"
 }
 
+// ENDS: also the end cell of every pair (anyseq_score_batch_ends).  Semiglobal: lane `outlane` keeps the first row
+// of the last column's maximum (strict '>'), the warp takes the first column of the last row's maximum, and
+// semiglobal_end applies the caller's precedence.  Local: pairs run with the subject as columns and the cells track
+// the lane's first maximum in its own row-major order (Cell TRACK); the warp takes the lowest (row, column) among
+// the lanes holding the maximum -- the first maximum of the matrix in row-major order (see batch_align.cu).
+template <int MODE, bool AFFINE, int K, bool MASK>
+__global__ void __launch_bounds__(kThreads, (K >= 32 ? 4 : (K >= 16 ? 5 : 6))) batch_ends_kernel(const BatchArgs a)
+{
+    constexpr bool ENDS = true;
+#include "batch_kernel_body.inl"
+}
 
-template <int MODE, bool AFFINE>
+template <int MODE, bool AFFINE, bool ENDS>
 static BatchKernelFn pick_batch_kernel_k(int K, bool mask)
 {
+#define ANYSEQ_PICK(KK, M) return ENDS ? batch_ends_kernel<MODE, AFFINE, KK, M> : batch_kernel<MODE, AFFINE, KK, M>
     if (mask) {
         switch (K) {
-            case 4: return batch_kernel<MODE, AFFINE, 4, true>;
-            case 8: return batch_kernel<MODE, AFFINE, 8, true>;
-            case 16: return batch_kernel<MODE, AFFINE, 16, true>;
-            case 32: return batch_kernel<MODE, AFFINE, 32, true>;
+            case 4: ANYSEQ_PICK(4, true);
+            case 8: ANYSEQ_PICK(8, true);
+            case 16: ANYSEQ_PICK(16, true);
+            case 32: ANYSEQ_PICK(32, true);
         }
     } else {
         switch (K) {
-            case 4: return batch_kernel<MODE, AFFINE, 4, false>;
-            case 8: return batch_kernel<MODE, AFFINE, 8, false>;
-            case 16: return batch_kernel<MODE, AFFINE, 16, false>;
+            case 4: ANYSEQ_PICK(4, false);
+            case 8: ANYSEQ_PICK(8, false);
+            case 16: ANYSEQ_PICK(16, false);
         }
     }
+#undef ANYSEQ_PICK
     return nullptr;
 }
 
-static BatchKernelFn pick_batch_kernel(int mode, bool affine, int K, bool mask)
+template <int MODE>
+static BatchKernelFn pick_batch_kernel_mode(bool affine, int K, bool mask, bool ends)
+{
+    if (ends) return affine ? pick_batch_kernel_k<MODE, true, true>(K, mask) : pick_batch_kernel_k<MODE, false, true>(K, mask);
+    return affine ? pick_batch_kernel_k<MODE, true, false>(K, mask) : pick_batch_kernel_k<MODE, false, false>(K, mask);
+}
+
+static BatchKernelFn pick_batch_kernel(int mode, bool affine, int K, bool mask, bool ends)
 {
     switch (mode) {
-        case kGlobal: return affine ? pick_batch_kernel_k<kGlobal, true>(K, mask) : pick_batch_kernel_k<kGlobal, false>(K, mask);
-        case kSemiglobal: return affine ? pick_batch_kernel_k<kSemiglobal, true>(K, mask) : pick_batch_kernel_k<kSemiglobal, false>(K, mask);
-        default: return affine ? pick_batch_kernel_k<kLocal, true>(K, mask) : pick_batch_kernel_k<kLocal, false>(K, mask);
+        case kGlobal: return pick_batch_kernel_mode<kGlobal>(affine, K, mask, ends);
+        case kSemiglobal: return pick_batch_kernel_mode<kSemiglobal>(affine, K, mask, ends);
+        default: return pick_batch_kernel_mode<kLocal>(affine, K, mask, ends);
     }
 }
 
-// Chooses the batch kernel for pairs of at most (max_long, max_short) symbols (alphabet already analysed: use_mask_,
-// ncodes_) and launches it on `st`; ba carries the input description and the score array.
+// Chooses the batch kernel for pairs of at most (max_long, max_short) symbols, queries of at most max_q and subjects
+// of at most max_s (alphabet already analysed: use_mask_, ncodes_) and launches it on `st`; ba carries the input
+// description, the score array and, when ba.ends is set, the end-cell array (the _ends kernels).
 int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool affine, BatchArgs& ba, int max_long,
-                         int max_short, cudaStream_t st)
+                         int max_short, int max_q, int max_s, cudaStream_t st)
 {
     const long long npairs = ba.npairs;
     // the bound is symmetric in the lengths and grows with both: the longest pair lengths bound every pair
     const int rc = check_score_range(sc, max_long, max_short);
     if (rc) return rc;
     const int limit = use_mask_ ? 1024 : 512;
+    const bool ends = ba.ends != nullptr;
+    // local end cells follow the row-major order of (query, subject), so those pairs always run with the subject as
+    // columns (the kernels ignore cols_longer then)
+    const bool subject_cols = ends && sc.mode == ANYSEQ_LOCAL;
     int cols_longer, ncols;
-    if (max_long <= limit) { cols_longer = 1; ncols = max_long; }
+    if (subject_cols) {
+        if (max_s > limit) {
+            char buf[240];
+            std::snprintf(buf, sizeof(buf), "batch end cells of local alignments: a subject of %d symbols is longer than %d; "
+                          "score such pairs with anyseq_score and the local_end_cell option", max_s, limit);
+            set_last_error(buf);
+            return ANYSEQ_ERR_UNSUPPORTED;
+        }
+        cols_longer = 0;
+        ncols = max_s;
+    } else if (max_long <= limit) { cols_longer = 1; ncols = max_long; }
     else if (max_short <= limit) { cols_longer = 0; ncols = max_short; }
     else {
         set_last_error("batch kernel: every pair needs one sequence of at most 1024 symbols (512 for large alphabets); "
@@ -251,7 +150,7 @@ int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool a
     int bias = 0;
     bool packed = false;
     if (use_mask_ && tune.batch_packed) {
-        const long long rows_max = cols_longer ? max_short : max_long;
+        const long long rows_max = subject_cols ? max_q : cols_longer ? max_short : max_long;
         const long long cols_pad = 32LL * K;
         const long long go = affine ? sp.gap_open : 0;
         const long long hmin = 2LL * sc.gap_init + (rows_max + cols_pad + 2) * sc.gap_extend;
@@ -265,13 +164,28 @@ int Engine::launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool a
     const bool quad = packed && tune.batch_quad && ncols <= 512;
     const int lanes = quad ? 16 : 32;     // lanes per group; a packed group relaxes two pairs
     if (quad) K = 32;
-    BatchKernelFn fn = packed ? pick_batch_x2_kernel(sc.mode, affine, K, lanes) : pick_batch_kernel(sc.mode, affine, K, use_mask_);
+    BatchKernelFn fn = packed ? pick_batch_x2_kernel(sc.mode, affine, K, lanes, ends)
+                              : pick_batch_kernel(sc.mode, affine, K, use_mask_, ends);
     if (!fn) { set_last_error("no batch kernel for this configuration"); return ANYSEQ_ERR_UNSUPPORTED; }
     // one column-mask set per pair of a warp, W words per lane, code and row; packed kernels spread the match bits to
     // every other bit (2 K bits per lane and row)
     const int W = packed ? (2 * K + 31) / 32 : 1;
     const int pairs_per_warp = packed ? 2 * (32 / lanes) : 1;
     const size_t dyn = use_mask_ ? sizeof(unsigned) * lanes * W * (size_t)ncodes_ * pairs_per_warp * kWarpsPerBlock : 0;
+    if (ends) {
+        // the local 16-bit ends kernels keep a row per lane and half in static shared memory (up to 32 KiB a block);
+        // with the column masks of a larger alphabet the block then needs more than the default 48 KiB, so these
+        // kernels may take up to the opt-in limit (the same value from every caller: no call lowers another's)
+        cudaFuncAttributes fa;
+        ANYSEQ_CUDA_CHECK(cudaFuncGetAttributes(&fa, fn));
+        if (fa.sharedSizeBytes + dyn > (size_t)(48 << 10)) {
+            int optin = 0;
+            ANYSEQ_CUDA_CHECK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+            if ((size_t)optin > fa.sharedSizeBytes)
+                ANYSEQ_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                       optin - (int)fa.sharedSizeBytes));
+        }
+    }
     int nb = 0;
     ANYSEQ_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, kThreads, dyn));
     if (nb < 1) { set_last_error("batch kernel does not fit on an SM"); return ANYSEQ_ERR_UNSUPPORTED; }
@@ -333,7 +247,7 @@ int Engine::batch_epilogue(int launches, anyseq_result* out)
 
 int Engine::score_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, const int64_t* d_qoff,
                                const uint8_t* d_s, const int64_t* d_soff, int64_t npairs, int32_t* d_scores,
-                               anyseq_result* out)
+                               anyseq_result* out, int32_t* d_ends)
 {
     std::lock_guard<std::recursive_mutex> lock(mu_);
     ANYSEQ_CUDA_CHECK(cudaSetDevice(device));
@@ -350,14 +264,15 @@ int Engine::score_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, con
     ba.soff = reinterpret_cast<const long long*>(d_soff);
     ba.npairs = npairs;
     ba.scores = d_scores;
+    ba.ends = d_ends;
     // totals (for the alphabet scan) and length statistics
     long long tot[2] = {0, 0};
     ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(&tot[0], d_qoff + npairs, sizeof(long long), cudaMemcpyDeviceToHost, stream_));
     ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(&tot[1], d_soff + npairs, sizeof(long long), cudaMemcpyDeviceToHost, stream_));
-    int max_long, max_short;
-    if ((rc = batch_len_stats(ba, &max_long, &max_short))) return rc;
+    int max_long, max_short, max_q, max_s;
+    if ((rc = batch_len_stats(ba, &max_long, &max_short, &max_q, &max_s))) return rc;
     if ((rc = analyse_alphabet(d_q, tot[0], d_s, tot[1]))) return rc;
-    if ((rc = launch_batch(sc, sp, affine, ba, max_long, max_short, stream_))) return rc;
+    if ((rc = launch_batch(sc, sp, affine, ba, max_long, max_short, max_q, max_s, stream_))) return rc;
     return batch_epilogue(5, out);
 }
 

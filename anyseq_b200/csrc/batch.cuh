@@ -28,6 +28,9 @@ struct BatchArgs {
     const int* slen;
     int qlen_u, slen_u;
     long long qstride, sstride;
+    // end cells (the _ends kernels): ends[2p] = end_i, ends[2p + 1] = end_j of pair p in the caller's coordinates.
+    // Last member, so that the parameter offsets of the score-only kernels stay where they were.
+    int* ends;
 };
 
 // where pair p's sequences start (symbol offset, or byte offset for 2-bit input) and how many symbols they have
@@ -68,9 +71,34 @@ __device__ __forceinline__ T pick_column(const T (&X)[K], int idx)
     return v;
 }
 
+// minimum over the lanes of a group of LANES lanes (a warp or a half-warp)
+template <int LANES>
+__device__ __forceinline__ int group_min(int v)
+{
+#pragma unroll
+    for (int o = LANES / 2; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+
+// Semiglobal end cell in the caller's coordinates, by the rule of finish_score_kernel (src/scoring.impala:51-63): the
+// caller's last row first (lowest j, the j = -1 candidate of value 0 winning ties), then its last column only if
+// strictly greater (lowest i).  (rv, rj): maximum of the kernel's last row and its first column; (cv, ci): maximum
+// of the kernel's last column and its first row.  With q_is_cols the kernel's rows are the subject, so its last
+// column is the caller's last row.
+__device__ __forceinline__ void semiglobal_end(int rv, int rj, int cv, int ci, bool q_is_cols, int lq, int ls, int& ei,
+                                               int& ej)
+{
+    int fv = q_is_cols ? cv : rv, fx = q_is_cols ? ci : rj;     // the caller's last row: (value, j)
+    int sv = q_is_cols ? rv : cv, sx = q_is_cols ? rj : ci;     // the caller's last column: (value, i)
+    if (0 >= fv) { fv = 0; fx = -1; }
+    if (0 >= sv) { sv = 0; sx = -1; }
+    if (sv > fv) { ei = sx; ej = ls - 1; }
+    else { ei = lq - 1; ej = fx; }
+}
+
 using BatchKernelFn = void (*)(const BatchArgs);
 // packed 16-bit kernels (batch_x2.cu): two pairs per group of `lanes` lanes (32: K = 4, 8, 16, 32; 16: K = 32, four
-// pairs per warp); nullptr for other combinations
-BatchKernelFn pick_batch_x2_kernel(int mode, bool affine, int K, int lanes);
+// pairs per warp); nullptr for other combinations.  ends: the kernels that also write end cells.
+BatchKernelFn pick_batch_x2_kernel(int mode, bool affine, int K, int lanes, bool ends);
 
 }  // namespace anyseq

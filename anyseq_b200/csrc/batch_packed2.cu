@@ -38,7 +38,7 @@ int Engine::use_2bit_alphabet()
     return lut_.ensure(512 + 64 + 16) ? ANYSEQ_ERR_NO_DEVICE : ANYSEQ_OK;
 }
 
-static void fill_args(BatchArgs& ba, const anyseq_packed_batch& b, int32_t* d_scores)
+static void fill_args(BatchArgs& ba, const anyseq_packed_batch& b, int32_t* d_scores, int32_t* d_ends)
 {
     std::memset(&ba, 0, sizeof(ba));
     ba.q = b.q2;
@@ -54,10 +54,11 @@ static void fill_args(BatchArgs& ba, const anyseq_packed_batch& b, int32_t* d_sc
     ba.packed2 = 1;
     ba.npairs = b.npairs;
     ba.scores = d_scores;
+    ba.ends = d_ends;
 }
 
 int Engine::score_batch_packed2_device(const anyseq_scoring& sc, const anyseq_packed_batch& b, int32_t* d_scores,
-                                       anyseq_result* out)
+                                       anyseq_result* out, int32_t* d_ends)
 {
     std::lock_guard<std::recursive_mutex> lock(mu_);
     ANYSEQ_CUDA_CHECK(cudaSetDevice(device));
@@ -69,20 +70,21 @@ int Engine::score_batch_packed2_device(const anyseq_scoring& sc, const anyseq_pa
     if (rc || b.npairs == 0) return rc;
     ANYSEQ_CUDA_CHECK(cudaEventRecord(ev0_, stream_));
     BatchArgs ba;
-    fill_args(ba, b, d_scores);
+    fill_args(ba, b, d_scores, d_ends);
     int max_long = std::max(b.q_len_uniform, b.s_len_uniform), max_short = std::min(b.q_len_uniform, b.s_len_uniform);
+    int max_q = b.q_len_uniform, max_s = b.s_len_uniform;
     int launches = 1;
     if (b.q_len || b.s_len) {
-        if ((rc = batch_len_stats(ba, &max_long, &max_short))) return rc;
+        if ((rc = batch_len_stats(ba, &max_long, &max_short, &max_q, &max_s))) return rc;
         launches += 1;
     }
     if ((rc = use_2bit_alphabet())) return rc;
-    if ((rc = launch_batch(sc, sp, affine, ba, max_long, max_short, stream_))) return rc;
+    if ((rc = launch_batch(sc, sp, affine, ba, max_long, max_short, max_q, max_s, stream_))) return rc;
     return batch_epilogue(launches, out);
 }
 
 int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_packed_batch& b, int32_t* scores,
-                                     anyseq_result* out)
+                                     anyseq_result* out, int32_t* ends)
 {
     std::lock_guard<std::recursive_mutex> lock(mu_);
     ANYSEQ_CUDA_CHECK(cudaSetDevice(device));
@@ -98,16 +100,20 @@ int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_pack
     auto slen = [&](int64_t p) { return b.s_len ? b.s_len[p] : b.s_len_uniform; };
     auto qbeg = [&](int64_t p) { return b.q_boff ? b.q_boff[p] : p * b.q_stride; };
     auto sbeg = [&](int64_t p) { return b.s_boff ? b.s_boff[p] : p * b.s_stride; };
-    int max_long = 0, max_short = 0;
+    int max_long = 0, max_short = 0, max_q = 0, max_s = 0;
     if (!b.q_len && !b.s_len) {
         max_long = std::max(b.q_len_uniform, b.s_len_uniform);
         max_short = std::min(b.q_len_uniform, b.s_len_uniform);
+        max_q = b.q_len_uniform;
+        max_s = b.s_len_uniform;
     } else {
         for (int64_t p = 0; p < np; ++p) {
             const int a = qlen(p), c = slen(p);
             if (a < 0 || c < 0) { set_last_error("packed batch: negative length"); return ANYSEQ_ERR_BAD_ARG; }
             max_long = std::max(max_long, std::max(a, c));
             max_short = std::max(max_short, std::min(a, c));
+            max_q = std::max(max_q, a);
+            max_s = std::max(max_s, c);
         }
     }
     if (b.q_boff || b.s_boff) {
@@ -135,7 +141,7 @@ int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_pack
     for (int64_t p0 = 0; p0 < np; p0 += chunk_pairs) {
         const int64_t p1 = std::min(np, p0 + chunk_pairs), n = p1 - p0;
         const size_t need = align16((size_t)(q_end(p1 - 1) - qbeg(p0))) + align16((size_t)(s_end(p1 - 1) - sbeg(p0))) +
-                            align16(sizeof(int32_t) * (size_t)n) +
+                            align16(sizeof(int32_t) * (size_t)n) + (ends ? align16(2 * sizeof(int32_t) * (size_t)n) : 0) +
                             (b.q_boff ? align16(sizeof(int64_t) * (size_t)n) : 0) + (b.s_boff ? align16(sizeof(int64_t) * (size_t)n) : 0) +
                             (b.q_len ? align16(sizeof(int32_t) * (size_t)n) : 0) + (b.s_len ? align16(sizeof(int32_t) * (size_t)n) : 0);
         slot_bytes = std::max(slot_bytes, need);
@@ -158,6 +164,8 @@ int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_pack
         uint8_t* d_q = base + off; off += align16(qbytes);
         uint8_t* d_s = base + off; off += align16(sbytes);
         int32_t* d_sc = reinterpret_cast<int32_t*>(base + off); off += align16(sizeof(int32_t) * (size_t)n);
+        int32_t* d_ends = nullptr;
+        if (ends) { d_ends = reinterpret_cast<int32_t*>(base + off); off += align16(2 * sizeof(int32_t) * (size_t)n); }
         ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(d_q, b.q2 + qb0, qbytes, cudaMemcpyHostToDevice, copy_stream_));
         ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(d_s, b.s2 + sb0, sbytes, cudaMemcpyHostToDevice, copy_stream_));
         h2d += (int64_t)(qbytes + sbytes);
@@ -181,10 +189,12 @@ int Engine::score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_pack
         ANYSEQ_CUDA_CHECK(cudaEventRecord(p2_ready_[slot], copy_stream_));
         ANYSEQ_CUDA_CHECK(cudaStreamWaitEvent(stream_, p2_ready_[slot], 0));
         BatchArgs ba;
-        fill_args(ba, d, d_sc);
-        rc = launch_batch(sc, sp, affine, ba, max_long, max_short, stream_);
+        fill_args(ba, d, d_sc, d_ends);
+        rc = launch_batch(sc, sp, affine, ba, max_long, max_short, max_q, max_s, stream_);
         if (rc) { cudaStreamSynchronize(copy_stream_); cudaStreamSynchronize(stream_); return rc; }
         ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(scores + p0, d_sc, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, stream_));
+        if (ends)
+            ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(ends + 2 * p0, d_ends, 2 * sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, stream_));
         ANYSEQ_CUDA_CHECK(cudaEventRecord(p2_done_[slot], stream_));
         launches += 1;
     }
@@ -214,6 +224,23 @@ int anyseq_score_batch_packed2_device(anyseq_ctx* ctx, const anyseq_scoring* sc,
 {
     if (!ctx || !sc || !device_batch) return ANYSEQ_ERR_BAD_ARG;
     return ctx->eng.score_batch_packed2_device(*sc, *device_batch, d_scores, out);
+}
+
+
+int anyseq_score_batch_packed2_ends(anyseq_ctx* ctx, const anyseq_scoring* sc, const anyseq_packed_batch* host_batch,
+                                    int32_t* scores, int32_t* ends, anyseq_result* out)
+{
+    if (!ctx || !sc || !host_batch || !ends) { anyseq::set_last_error("packed batch: null argument"); return ANYSEQ_ERR_BAD_ARG; }
+    return ctx->eng.score_batch_packed2_host(*sc, *host_batch, scores, out, ends);
+}
+
+
+int anyseq_score_batch_packed2_ends_device(anyseq_ctx* ctx, const anyseq_scoring* sc,
+                                           const anyseq_packed_batch* device_batch, int32_t* d_scores, int32_t* d_ends,
+                                           anyseq_result* out)
+{
+    if (!ctx || !sc || !device_batch || !d_ends) { anyseq::set_last_error("packed batch: null argument"); return ANYSEQ_ERR_BAD_ARG; }
+    return ctx->eng.score_batch_packed2_device(*sc, *device_batch, d_scores, out, d_ends);
 }
 
 

@@ -6,7 +6,7 @@
 // straight into it, or copying from caller memory), submit() starts the H2D
 // copies on the stream's own copy stream, and the consumer's collect() runs
 // the batch kernel of that chunk on the engine's stream and brings the scores
-// back.  Filling and copying chunk c+1 therefore overlap the kernel of chunk c;
+// back (and the end cells of its pairs, for a stream opened with ends).  Filling and copying chunk c+1 therefore overlap the kernel of chunk c;
 // no slot is touched by two stages at once (free -> filling -> submitted ->
 // done -> free).  The reference's reader offers the same producer/consumer
 // split on the host (next()/skip() under a mutex, src/sequence_io.cpp:13-41);
@@ -46,8 +46,8 @@ struct PinnedBuffer {
 
 struct BatchSlot {
     enum State { kFree, kFilling, kSubmitted, kDone } state = kFree;
-    PinnedBuffer hq, hs, hqo, hso, hscores;
-    DeviceBuffer dq, ds, dqo, dso, dscores;
+    PinnedBuffer hq, hs, hqo, hso, hscores, hends;
+    DeviceBuffer dq, ds, dqo, dso, dscores, dends;      // hends / dends: streams opened with ends only
     cudaEvent_t ready = nullptr;     // H2D of this slot's chunk has finished
     int64_t npairs = 0;
     float kernel_ms = 0.f;
@@ -56,13 +56,14 @@ struct BatchSlot {
 
 class BatchStream {
 public:
-    BatchStream(Engine* eng, const anyseq_scoring& sc) : eng_(eng), sc_(sc) {}
+    BatchStream(Engine* eng, const anyseq_scoring& sc, bool ends) : eng_(eng), sc_(sc), ends_(ends) {}
     ~BatchStream() { destroy(); }
 
-    // reuse of an idle stream (every slot free) for another batch: pinned allocations are expensive
-    bool reusable(int64_t cap_pairs, int64_t cap_q, int64_t cap_s) const
+    // reuse of an idle stream (every slot free) for another batch: pinned allocations are expensive.  A stream with
+    // ends runs the _ends kernels, which orient local pairs differently, so it serves only calls that want ends.
+    bool reusable(int64_t cap_pairs, int64_t cap_q, int64_t cap_s, bool ends) const
     {
-        return !slots_.empty() && !failed_ && cap_pairs <= cap_pairs_ && cap_q <= cap_q_ && cap_s <= cap_s_;
+        return !slots_.empty() && !failed_ && cap_pairs <= cap_pairs_ && cap_q <= cap_q_ && cap_s <= cap_s_ && ends_ == ends;
     }
     void restart(const anyseq_scoring& sc)
     {
@@ -89,12 +90,12 @@ public:
         const size_t no = sizeof(int64_t) * (size_t)(cap_pairs_ + 1), ns = sizeof(int32_t) * (size_t)cap_pairs_;
         for (BatchSlot& s : slots_) {
             if (s.hq.ensure((size_t)cap_q_) || s.hs.ensure((size_t)cap_s_) || s.hqo.ensure(no) || s.hso.ensure(no) ||
-                s.hscores.ensure(ns)) {
+                s.hscores.ensure(ns) || (ends_ && s.hends.ensure(2 * ns))) {
                 set_last_error("batch stream: out of pinned host memory");
                 return ANYSEQ_ERR_NO_DEVICE;
             }
             if (s.dq.ensure((size_t)cap_q_ + 64) || s.ds.ensure((size_t)cap_s_ + 64) || s.dqo.ensure(no) || s.dso.ensure(no) ||
-                s.dscores.ensure(ns))
+                s.dscores.ensure(ns) || (ends_ && s.dends.ensure(2 * ns)))
                 return ANYSEQ_ERR_NO_DEVICE;
             ANYSEQ_CUDA_CHECK(cudaEventCreateWithFlags(&s.ready, cudaEventDisableTiming));
         }
@@ -106,8 +107,8 @@ public:
         if (eng_ && eng_->device >= 0) cudaSetDevice(eng_->device);
         if (copy_stream_) cudaStreamSynchronize(copy_stream_);
         for (BatchSlot& s : slots_) {
-            s.hq.release(); s.hs.release(); s.hqo.release(); s.hso.release(); s.hscores.release();
-            s.dq.release(); s.ds.release(); s.dqo.release(); s.dso.release(); s.dscores.release();
+            s.hq.release(); s.hs.release(); s.hqo.release(); s.hso.release(); s.hscores.release(); s.hends.release();
+            s.dq.release(); s.ds.release(); s.dqo.release(); s.dso.release(); s.dscores.release(); s.dends.release();
             if (s.ready) cudaEventDestroy(s.ready);
             s.ready = nullptr;
         }
@@ -202,12 +203,16 @@ public:
         if (s.npairs > 0) {
             ANYSEQ_CUDA_CHECK(cudaStreamWaitEvent(eng_->stream(), s.ready, 0));
             int rc = eng_->score_batch_device(sc_, s.dq.as<uint8_t>(), s.dqo.as<int64_t>(), s.ds.as<uint8_t>(),
-                                              s.dso.as<int64_t>(), s.npairs, s.dscores.as<int32_t>(), &r);
+                                              s.dso.as<int64_t>(), s.npairs, s.dscores.as<int32_t>(), &r,
+                                              ends_ ? s.dends.as<int32_t>() : nullptr);
             if (rc) { fail(); return rc; }
             ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(s.hscores.ptr, s.dscores.ptr, sizeof(int32_t) * (size_t)s.npairs,
                                               cudaMemcpyDeviceToHost, eng_->stream()));
+            if (ends_)
+                ANYSEQ_CUDA_CHECK(cudaMemcpyAsync(s.hends.ptr, s.dends.ptr, 2 * sizeof(int32_t) * (size_t)s.npairs,
+                                                  cudaMemcpyDeviceToHost, eng_->stream()));
             ANYSEQ_CUDA_CHECK(cudaStreamSynchronize(eng_->stream()));
-            d2h_bytes_ += (long long)sizeof(int32_t) * s.npairs;
+            d2h_bytes_ += (long long)sizeof(int32_t) * s.npairs * (ends_ ? 3 : 1);
         }
         s.kernel_ms = r.kernel_ms;
         s.launches = r.kernel_launches;
@@ -223,6 +228,15 @@ public:
         c->kernel_ms = s.kernel_ms;
         c->slot = idx;
         return ANYSEQ_OK;
+    }
+
+    // consumer: the end cells of a collected chunk (2 per pair, pinned, valid until release); null without ends
+    const int32_t* chunk_ends(const anyseq_batch_chunk* c)
+    {
+        if (!ends_ || !c || c->slot < 0 || c->slot >= (int)slots_.size()) return nullptr;
+        std::lock_guard<std::mutex> lk(mu_);
+        const BatchSlot& s = slots_[(size_t)c->slot];
+        return s.state == BatchSlot::kDone ? static_cast<const int32_t*>(s.hends.ptr) : nullptr;
     }
 
     // consumer: scores of the chunk have been used, its slot may be refilled
@@ -257,6 +271,7 @@ public:
 private:
     Engine* eng_;
     anyseq_scoring sc_;
+    bool ends_;
     cudaStream_t copy_stream_ = nullptr;
     std::vector<BatchSlot> slots_;
     std::deque<int> order_;
@@ -288,7 +303,7 @@ static void parallel_copy(char* dst, const char* src, size_t n, int threads)
 }
 
 int Engine::score_batch_host(const anyseq_scoring& sc, const char* q, const int64_t* qoff, const char* s,
-                             const int64_t* soff, int64_t npairs, int32_t* scores, anyseq_result* out)
+                             const int64_t* soff, int64_t npairs, int32_t* scores, anyseq_result* out, int32_t* ends)
 {
     ScoreParams sp;
     bool affine;
@@ -312,13 +327,13 @@ int Engine::score_batch_host(const anyseq_scoring& sc, const char* q, const int6
     // one cached stream per engine: its pinned + device slots survive between calls
     std::lock_guard<std::recursive_mutex> lock(mu_);
     BatchStream* cached = static_cast<BatchStream*>(host_batch_stream_);
-    if (cached && !cached->reusable(cap_pairs, cap_q, cap_s)) {
+    if (cached && !cached->reusable(cap_pairs, cap_q, cap_s, ends != nullptr)) {
         delete cached;
         cached = nullptr;
         host_batch_stream_ = nullptr;
     }
     if (!cached) {
-        cached = new BatchStream(this, sc);
+        cached = new BatchStream(this, sc, ends != nullptr);
         rc = cached->init(std::max<int64_t>(cap_pairs, std::min<int64_t>(tune.batch_chunk_pairs, 1 << 18)), cap_q, cap_s, 3);
         if (rc) { delete cached; return rc; }
         host_batch_stream_ = cached;
@@ -354,6 +369,7 @@ int Engine::score_batch_host(const anyseq_scoring& sc, const char* q, const int6
         crc = st.collect(&c);
         if (crc != ANYSEQ_OK) break;
         std::memcpy(scores + done, c.scores, sizeof(int32_t) * (size_t)c.npairs);
+        if (ends) std::memcpy(ends + 2 * done, st.chunk_ends(&c), 2 * sizeof(int32_t) * (size_t)c.npairs);
         done += c.npairs;
         st.release(&c);
     }
@@ -385,10 +401,8 @@ struct anyseq_batch_stream {
     anyseq::BatchStream* impl;
 };
 
-extern "C" {
-
-int anyseq_batch_stream_open(anyseq_ctx* ctx, const anyseq_scoring* sc, int64_t cap_pairs, int64_t cap_query_bytes,
-                             int64_t cap_subject_bytes, int slots, anyseq_batch_stream** out)
+static int open_stream(anyseq_ctx* ctx, const anyseq_scoring* sc, int64_t cap_pairs, int64_t cap_query_bytes,
+                       int64_t cap_subject_bytes, int slots, bool ends, anyseq_batch_stream** out)
 {
     if (!ctx || !sc || !out || cap_pairs < 1 || cap_query_bytes < 1 || cap_subject_bytes < 1) {
         anyseq::set_last_error("batch stream: bad arguments");
@@ -399,11 +413,30 @@ int anyseq_batch_stream_open(anyseq_ctx* ctx, const anyseq_scoring* sc, int64_t 
     bool affine;
     int rc = anyseq::make_score_params(*sc, &sp, &affine);
     if (rc) return rc;
-    anyseq::BatchStream* impl = new anyseq::BatchStream(&ctx->eng, *sc);
+    anyseq::BatchStream* impl = new anyseq::BatchStream(&ctx->eng, *sc, ends);
     rc = impl->init(cap_pairs, cap_query_bytes, cap_subject_bytes, slots <= 0 ? 3 : slots);
     if (rc) { delete impl; return rc; }
     *out = new anyseq_batch_stream{impl};
     return ANYSEQ_OK;
+}
+
+extern "C" {
+
+int anyseq_batch_stream_open(anyseq_ctx* ctx, const anyseq_scoring* sc, int64_t cap_pairs, int64_t cap_query_bytes,
+                             int64_t cap_subject_bytes, int slots, anyseq_batch_stream** out)
+{
+    return open_stream(ctx, sc, cap_pairs, cap_query_bytes, cap_subject_bytes, slots, false, out);
+}
+
+int anyseq_batch_stream_open_ends(anyseq_ctx* ctx, const anyseq_scoring* sc, int64_t cap_pairs, int64_t cap_query_bytes,
+                                  int64_t cap_subject_bytes, int slots, anyseq_batch_stream** out)
+{
+    return open_stream(ctx, sc, cap_pairs, cap_query_bytes, cap_subject_bytes, slots, true, out);
+}
+
+const int32_t* anyseq_batch_stream_chunk_ends(anyseq_batch_stream* st, const anyseq_batch_chunk* chunk)
+{
+    return st ? st->impl->chunk_ends(chunk) : nullptr;
 }
 
 int anyseq_batch_stream_acquire(anyseq_batch_stream* st, anyseq_batch_chunk* chunk)

@@ -36,7 +36,8 @@ struct X2State {
     unsigned tm[W];      // match bits of the lane's row: bit 2c = pair A column c, bit 2c+1 = pair B
 };
 
-template <bool LOCAL, bool AFFINE, int K, int C>
+// ROWMAX (local end cells): s.best is the maximum of the lane's cells of this row only, not a running maximum
+template <bool LOCAL, bool AFFINE, int K, int C, bool ROWMAX = false>
 struct CellX2 {
     template <int KF, int W>
     static __device__ __forceinline__ void run(unsigned (&X)[K], unsigned (&F)[KF], X2State<W>& s, const X2Const& k)
@@ -56,13 +57,14 @@ struct CellX2 {
         }
         if constexpr (LOCAL) {
             h = __vmaxs2(h, k.floor2);
-            if constexpr ((C & 1) != 0) s.best = __vimax3_s16x2(s.best, h, s.hprev);
+            if constexpr (ROWMAX && C == 1) s.best = __vmaxs2(s.hprev, h);
+            else if constexpr ((C & 1) != 0) s.best = __vimax3_s16x2(s.best, h, s.hprev);
             else s.hprev = h;
         }
         const unsigned x = AFFINE ? (unsigned)imad_add((int)h, k.one, k.go_c) : h;
         X[C] = x;
         s.xleft = x;
-        if constexpr (C + 1 < K) CellX2<LOCAL, AFFINE, K, C + 1>::run(X, F, s, k);
+        if constexpr (C + 1 < K) CellX2<LOCAL, AFFINE, K, C + 1, ROWMAX>::run(X, F, s, k);
     }
 };
 
@@ -82,6 +84,23 @@ __device__ __forceinline__ void max_column_u(unsigned& best, const unsigned (&X)
     }
 }
 
+// X[idx] for a warp-uniform run-time idx, by the same kind of jump as max_column_u
+template <int K>
+__device__ __forceinline__ unsigned column_u(const unsigned (&X)[K], int idx)
+{
+    unsigned v = 0u;
+    switch (idx) {
+#define ANYSEQ_CASE(c) case c: if constexpr (c < K) v = X[c < K ? c : 0]; break;
+        ANYSEQ_CASE(0) ANYSEQ_CASE(1) ANYSEQ_CASE(2) ANYSEQ_CASE(3) ANYSEQ_CASE(4) ANYSEQ_CASE(5) ANYSEQ_CASE(6) ANYSEQ_CASE(7)
+        ANYSEQ_CASE(8) ANYSEQ_CASE(9) ANYSEQ_CASE(10) ANYSEQ_CASE(11) ANYSEQ_CASE(12) ANYSEQ_CASE(13) ANYSEQ_CASE(14) ANYSEQ_CASE(15)
+        ANYSEQ_CASE(16) ANYSEQ_CASE(17) ANYSEQ_CASE(18) ANYSEQ_CASE(19) ANYSEQ_CASE(20) ANYSEQ_CASE(21) ANYSEQ_CASE(22) ANYSEQ_CASE(23)
+        ANYSEQ_CASE(24) ANYSEQ_CASE(25) ANYSEQ_CASE(26) ANYSEQ_CASE(27) ANYSEQ_CASE(28) ANYSEQ_CASE(29) ANYSEQ_CASE(30) ANYSEQ_CASE(31)
+#undef ANYSEQ_CASE
+        default: break;
+    }
+    return v;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // batch_pairs: two pairs per group of LANES lanes, relaxed together in the two halves of every register.
 //   LANES = 32: a group is the warp, two pairs per warp, K = 4..32 columns per lane.
@@ -89,16 +108,26 @@ __device__ __forceinline__ void max_column_u(unsigned& best, const unsigned (&X)
 //   skew of a work item is 15 steps instead of 31: a 150-row read costs 165 instead of 181 steps (the 17 % fill/drain
 //   of 32 lanes becomes 9 %).  Used when the column sequences have at most 512 symbols (BASELINE configs[3]: 500 bp
 //   windows).
+// ENDS: also the end cell of every pair (anyseq_score_batch_ends), per half:
+//   semiglobal: lane `outlane` keeps the first row of the last column's maximum (strict '>'); at the end the group
+//     takes the first column of the last row's maximum and semiglobal_end applies the caller's precedence.
+//   local: pairs run with the subject as columns.  The cells fold into a per-row maximum; when it beats the lane's
+//     maximum, the lane notes the row and stores its K cells to shared memory (one slot per half), and at the end the
+//     group takes the first maximum in row-major order: the lowest row among the lanes holding the maximum, then the
+//     lowest column holding it in the stored rows of those lanes.
 // ---------------------------------------------------------------------------------------------------------------
-template <int MODE, bool AFFINE, int K, int LANES>
+template <int MODE, bool AFFINE, int K, int LANES, bool ENDS = false>
 __device__ __forceinline__ void batch_pairs(const BatchArgs& a)
 {
     static_assert(LANES == 32 || LANES == 16, "a group is a warp or a half-warp");
     constexpr int G = 32 / LANES;                     // groups per warp; a work item is 2 G consecutive pairs
     constexpr bool LOCAL = MODE == kLocal;
     constexpr bool GLOB = MODE == kGlobal;
+    constexpr bool LOCAL_ENDS = ENDS && LOCAL;
     __shared__ uint8_t s_rows[kWarpsPerBlock][G][2][64];
     __shared__ uint8_t s_lut[256];
+    // LOCAL_ENDS: the row of each lane's maximum of pair A / B, as [warp][half][K / 4][lane] groups of four cells
+    __shared__ uint4 s_snap[LOCAL_ENDS ? kWarpsPerBlock * 2 * (K / 4) * 32 : 1];
     extern __shared__ unsigned s_dyn[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int grp = lane / LANES, gl = lane % LANES;  // the lane's group and its lane within the group
@@ -153,10 +182,11 @@ __device__ __forceinline__ void batch_pairs(const BatchArgs& a)
             const int lq = batch_q_len(a, pa), ls = batch_s_len(a, pa);
             const bool empty = lq == 0 || ls == 0;
             int scoreA, scoreB;
+            int eiA = lq - 1, ejA = ls - 1, eiB = lq - 1, ejB = ls - 1;     // end cells: global and empty pairs
             if (G == 1 && empty) {
                 scoreA = scoreB = empty_pair_score<MODE>(a, lq, ls);     // a warp-wide group skips the DP
             } else {
-                const bool q_is_cols = a.cols_longer ? (lq >= ls) : (lq < ls);
+                const bool q_is_cols = LOCAL_ENDS ? false : (a.cols_longer ? (lq >= ls) : (lq < ls));
                 const uint8_t* colsA = q_is_cols ? a.q + qa0 : a.s + sa0;
                 const uint8_t* rowsA = q_is_cols ? a.s + sa0 : a.q + qa0;
                 const uint8_t* colsB = q_is_cols ? a.q + qb0 : a.s + sb0;
@@ -202,6 +232,15 @@ __device__ __forceinline__ void batch_pairs(const BatchArgs& a)
                 const int outlane = live ? (n - 1) / K : 0, outc = live ? (n - 1) % K : 0;
                 unsigned hr = 0, er = 0;
                 unsigned colbest = pack2(kNeg16, kNeg16);    // semiglobal: max over H(i, n-1), kept by lane `outlane`
+                int ciA = 0, ciB = 0;                        // ENDS semiglobal: its first row, per half
+                unsigned lbest = k.floor2;                   // LOCAL_ENDS: the lane's maximum ...
+                int rowA = 0, rowB = 0;                      // ... and the first row holding it, per half
+                uint4* snap = s_snap + (LOCAL_ENDS ? (warp * 2 * (K / 4) * 32 + lane) : 0);
+                auto store_row = [&](int half) {
+#pragma unroll
+                    for (int w = 0; w < K / 4; ++w)
+                        snap[(half * (K / 4) + w) * 32] = make_uint4(X[4 * w], X[4 * w + 1], X[4 * w + 2], X[4 * w + 3]);
+                };
                 X2State<W> st;
                 st.dd = 0; st.e = 0; st.xleft = 0;
 #pragma unroll
@@ -240,11 +279,28 @@ __device__ __forceinline__ void batch_pairs(const BatchArgs& a)
                             dcarry = xl;
                             st.xleft = xl;
                             st.e = el;
-                            CellX2<LOCAL, AFFINE, K, 0>::run(X, F, st, k);
+                            CellX2<LOCAL, AFFINE, K, 0, LOCAL_ENDS>::run(X, F, st, k);
                             hr = st.xleft;
                             er = st.e;
-                            if constexpr (MODE == kSemiglobal) {
+                            if constexpr (MODE == kSemiglobal && ENDS) {
+                                if (gl == outlane) {
+                                    const unsigned nb = __vmaxs2(colbest, column_u<K>(X, outc));
+                                    const unsigned d = nb ^ colbest;     // halves that grew strictly
+                                    if (d & 0xffffu) ciA = i;
+                                    if (d >> 16) ciB = i;
+                                    colbest = nb;
+                                }
+                            } else if constexpr (MODE == kSemiglobal) {
                                 if (gl == outlane) max_column_u<K>(colbest, X, outc);
+                            }
+                            if constexpr (LOCAL_ENDS) {
+                                const unsigned nb = __vmaxs2(lbest, st.best);
+                                if (nb != lbest) {
+                                    const unsigned d = nb ^ lbest;
+                                    if (d & 0xffffu) { rowA = i; store_row(0); }
+                                    if (d >> 16) { rowB = i; store_row(1); }
+                                    lbest = nb;
+                                }
                             }
                         }
 #pragma unroll
@@ -256,6 +312,30 @@ __device__ __forceinline__ void batch_pairs(const BatchArgs& a)
                     const unsigned v = __shfl_sync(kFull, pick_column(X, outc), outlane, LANES);
                     scoreA = lo16(v) - go - bias;
                     scoreB = hi16(v) - go - bias;
+                } else if constexpr (MODE == kSemiglobal && ENDS) {
+                    // the kernel's last row: its maximum, then the first column holding it, per half
+                    unsigned rbest = pack2(kNeg16, kNeg16);
+#pragma unroll
+                    for (int c = 0; c < K; ++c)
+                        if (jl + c < n) rbest = __vmaxs2(rbest, X[c]);
+#pragma unroll
+                    for (int o = LANES / 2; o > 0; o >>= 1) rbest = __vmaxs2(rbest, __shfl_xor_sync(kFull, rbest, o));
+                    int rjA = 0x7fffffff, rjB = 0x7fffffff;
+#pragma unroll
+                    for (int c = K - 1; c >= 0; --c) {
+                        if (jl + c < n && lo16(X[c]) == lo16(rbest)) rjA = jl + c;
+                        if (jl + c < n && hi16(X[c]) == hi16(rbest)) rjB = jl + c;
+                    }
+                    rjA = group_min<LANES>(rjA);
+                    rjB = group_min<LANES>(rjB);
+                    const unsigned cb = __shfl_sync(kFull, colbest, outlane, LANES);
+                    const int cA = __shfl_sync(kFull, ciA, outlane, LANES), cB = __shfl_sync(kFull, ciB, outlane, LANES);
+                    const int rvA = lo16(rbest) - go - bias, rvB = hi16(rbest) - go - bias;
+                    const int cvA = lo16(cb) - go - bias, cvB = hi16(cb) - go - bias;
+                    scoreA = max(max(rvA, cvA), 0);                              // candidates H(m-1,-1) = H(-1,n-1) = 0
+                    scoreB = max(max(rvB, cvB), 0);
+                    semiglobal_end(rvA, rjA, cvA, cA, q_is_cols, lq, ls, eiA, ejA);
+                    semiglobal_end(rvB, rjB, cvB, cB, q_is_cols, lq, ls, eiB, ejB);
                 } else if constexpr (MODE == kSemiglobal) {
                     unsigned best = colbest;
 #pragma unroll
@@ -265,6 +345,37 @@ __device__ __forceinline__ void batch_pairs(const BatchArgs& a)
                     for (int o = LANES / 2; o > 0; o >>= 1) best = __vmaxs2(best, __shfl_xor_sync(kFull, best, o));
                     scoreA = max(lo16(best) - go - bias, 0);                     // candidates H(m-1,-1) = H(-1,n-1) = 0
                     scoreB = max(hi16(best) - go - bias, 0);
+                } else if constexpr (LOCAL_ENDS) {
+                    unsigned best = lbest;
+#pragma unroll
+                    for (int o = LANES / 2; o > 0; o >>= 1) best = __vmaxs2(best, __shfl_xor_sync(kFull, best, o));
+                    scoreA = lo16(best) - bias;
+                    scoreB = hi16(best) - bias;
+                    // the first row holding the maximum, then the first column of that row holding it (rows without a
+                    // positive cell: the maximum 0 is first reached at (0, 0))
+                    const bool hasA = lo16(lbest) == lo16(best), hasB = hi16(lbest) == hi16(best);
+                    const int riA = group_min<LANES>(hasA ? rowA : 0x7fffffff);
+                    const int riB = group_min<LANES>(hasB ? rowB : 0x7fffffff);
+                    int cjA = 0x7fffffff, cjB = 0x7fffffff;
+                    const int tA = lo16(best) + go, tB = hi16(best) + go;        // stored cells are X = H (+ go)
+                    if (hasA && rowA == riA && scoreA > 0) {
+                        for (int c = K - 1; c >= 0; --c) {
+                            const uint4 v = snap[(c / 4) * 32];
+                            const unsigned x = (c & 3) == 0 ? v.x : (c & 3) == 1 ? v.y : (c & 3) == 2 ? v.z : v.w;
+                            if (lo16(x) == tA) cjA = jl + c;
+                        }
+                    }
+                    if (hasB && rowB == riB && scoreB > 0) {
+                        for (int c = K - 1; c >= 0; --c) {
+                            const uint4 v = snap[(K / 4 + c / 4) * 32];
+                            const unsigned x = (c & 3) == 0 ? v.x : (c & 3) == 1 ? v.y : (c & 3) == 2 ? v.z : v.w;
+                            if (hi16(x) == tB) cjB = jl + c;
+                        }
+                    }
+                    cjA = group_min<LANES>(cjA);
+                    cjB = group_min<LANES>(cjB);
+                    eiA = scoreA > 0 ? riA : 0; ejA = scoreA > 0 ? cjA : 0;
+                    eiB = scoreB > 0 ? riB : 0; ejB = scoreB > 0 ? cjB : 0;
                 } else {
                     unsigned best = __vmaxs2(st.best, st.hprev);
 #pragma unroll
@@ -272,11 +383,20 @@ __device__ __forceinline__ void batch_pairs(const BatchArgs& a)
                     scoreA = lo16(best) - bias;
                     scoreB = hi16(best) - bias;
                 }
-                if (active && empty) scoreA = scoreB = empty_pair_score<MODE>(a, lq, ls);
+                if (active && empty) {
+                    scoreA = scoreB = empty_pair_score<MODE>(a, lq, ls);
+                    eiA = eiB = lq - 1;
+                    ejA = ejB = ls - 1;
+                }
             }
             if (active && gl == 0) {
                 a.scores[pa] = scoreA;
                 if (pb != pa) a.scores[pb] = scoreB;
+                if constexpr (ENDS) {
+                    a.ends[2 * pa] = eiA;
+                    a.ends[2 * pa + 1] = ejA;
+                    if (pb != pa) { a.ends[2 * pb] = eiB; a.ends[2 * pb + 1] = ejB; }
+                }
             }
         }
         unsigned long long nxt = 0;
@@ -299,25 +419,45 @@ __global__ void __launch_bounds__(kThreads, 3) batch_x4_kernel(const BatchArgs a
     batch_pairs<MODE, AFFINE, 32, 16>(a);
 }
 
+// the same two widths writing end cells as well (anyseq_score_batch_ends)
+template <int MODE, bool AFFINE, int K>
+__global__ void __launch_bounds__(kThreads, (K >= 32 ? 4 : (K >= 16 ? 5 : 6))) batch_x2_ends_kernel(const BatchArgs a)
+{
+    batch_pairs<MODE, AFFINE, K, 32, true>(a);
+}
+
 template <int MODE, bool AFFINE>
+__global__ void __launch_bounds__(kThreads, 3) batch_x4_ends_kernel(const BatchArgs a)
+{
+    batch_pairs<MODE, AFFINE, 32, 16, true>(a);
+}
+
+template <int MODE, bool AFFINE, bool ENDS>
 static BatchKernelFn pick_x2(int K, int lanes)
 {
-    if (lanes == 16) return K == 32 ? batch_x4_kernel<MODE, AFFINE> : nullptr;
+    if (lanes == 16) return K != 32 ? nullptr : ENDS ? batch_x4_ends_kernel<MODE, AFFINE> : batch_x4_kernel<MODE, AFFINE>;
     switch (K) {
-        case 4: return batch_x2_kernel<MODE, AFFINE, 4>;
-        case 8: return batch_x2_kernel<MODE, AFFINE, 8>;
-        case 16: return batch_x2_kernel<MODE, AFFINE, 16>;
-        case 32: return batch_x2_kernel<MODE, AFFINE, 32>;
+        case 4: return ENDS ? batch_x2_ends_kernel<MODE, AFFINE, 4> : batch_x2_kernel<MODE, AFFINE, 4>;
+        case 8: return ENDS ? batch_x2_ends_kernel<MODE, AFFINE, 8> : batch_x2_kernel<MODE, AFFINE, 8>;
+        case 16: return ENDS ? batch_x2_ends_kernel<MODE, AFFINE, 16> : batch_x2_kernel<MODE, AFFINE, 16>;
+        case 32: return ENDS ? batch_x2_ends_kernel<MODE, AFFINE, 32> : batch_x2_kernel<MODE, AFFINE, 32>;
     }
     return nullptr;
 }
 
-BatchKernelFn pick_batch_x2_kernel(int mode, bool affine, int K, int lanes)
+template <int MODE>
+static BatchKernelFn pick_x2_mode(bool affine, int K, int lanes, bool ends)
+{
+    if (ends) return affine ? pick_x2<MODE, true, true>(K, lanes) : pick_x2<MODE, false, true>(K, lanes);
+    return affine ? pick_x2<MODE, true, false>(K, lanes) : pick_x2<MODE, false, false>(K, lanes);
+}
+
+BatchKernelFn pick_batch_x2_kernel(int mode, bool affine, int K, int lanes, bool ends)
 {
     switch (mode) {
-        case kGlobal: return affine ? pick_x2<kGlobal, true>(K, lanes) : pick_x2<kGlobal, false>(K, lanes);
-        case kSemiglobal: return affine ? pick_x2<kSemiglobal, true>(K, lanes) : pick_x2<kSemiglobal, false>(K, lanes);
-        default: return affine ? pick_x2<kLocal, true>(K, lanes) : pick_x2<kLocal, false>(K, lanes);
+        case kGlobal: return pick_x2_mode<kGlobal>(affine, K, lanes, ends);
+        case kSemiglobal: return pick_x2_mode<kSemiglobal>(affine, K, lanes, ends);
+        default: return pick_x2_mode<kLocal>(affine, K, lanes, ends);
     }
 }
 

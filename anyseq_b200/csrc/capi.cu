@@ -209,6 +209,29 @@ int anyseq_score_batch_device(anyseq_ctx* ctx, const anyseq_scoring* sc, const v
                                        d_scores, out);
 }
 
+int anyseq_score_batch_ends(anyseq_ctx* ctx, const anyseq_scoring* sc, const char* queries, const int64_t* q_off,
+                            const char* subjects, const int64_t* s_off, int64_t npairs, int32_t* scores, int32_t* ends,
+                            anyseq_result* out)
+{
+    if (!ctx || !sc || !q_off || !s_off || !scores || !ends || npairs < 0) {
+        anyseq::set_last_error("batch end cells: null argument");
+        return ANYSEQ_ERR_BAD_ARG;
+    }
+    return ctx->eng.score_batch_host(*sc, queries, q_off, subjects, s_off, npairs, scores, out, ends);
+}
+
+int anyseq_score_batch_ends_device(anyseq_ctx* ctx, const anyseq_scoring* sc, const void* d_queries,
+                                   const int64_t* d_q_off, const void* d_subjects, const int64_t* d_s_off,
+                                   int64_t npairs, int32_t* d_scores, int32_t* d_ends, anyseq_result* out)
+{
+    if (!ctx || !sc || !d_q_off || !d_s_off || !d_scores || !d_ends || npairs < 0) {
+        anyseq::set_last_error("batch end cells: null argument");
+        return ANYSEQ_ERR_BAD_ARG;
+    }
+    return ctx->eng.score_batch_device(*sc, static_cast<const uint8_t*>(d_queries), d_q_off,
+                                       static_cast<const uint8_t*>(d_subjects), d_s_off, npairs, d_scores, out, d_ends);
+}
+
 int anyseq_strip_inbox_create(anyseq_ctx* ctx, int rows, anyseq_inbox** out, void* ipc_handle_64B)
 {
     if (!ctx || !out || rows < 1) return ANYSEQ_ERR_BAD_ARG;

@@ -115,12 +115,13 @@ public:
     // full-matrix traceback (traceback_full.cu); start2 = get_alignment_start()
     int align_full_host(const anyseq_scoring& sc, const char* q, int m, const char* s, int n,
                         char* alq, char* als, anyseq_result* out, int* start2);
+    // d_ends / ends (2 * npairs, may be null): end cells as anyseq_score gives them (the _ends batch kernels)
     int score_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, const int64_t* d_qoff,
                            const uint8_t* d_s, const int64_t* d_soff, int64_t npairs,
-                           int32_t* d_scores, anyseq_result* out);
+                           int32_t* d_scores, anyseq_result* out, int32_t* d_ends = nullptr);
     int score_batch_host(const anyseq_scoring& sc, const char* q, const int64_t* qoff,
                          const char* s, const int64_t* soff, int64_t npairs, int32_t* scores,
-                         anyseq_result* out);
+                         anyseq_result* out, int32_t* ends = nullptr);
     // full-matrix tracebacks of a batch of pairs with subjects of at most 1024 symbols (batch_align.cu): per pair what
     // align_full_host gives; ends / starts may be null
     int align_batch_device(const anyseq_scoring& sc, const uint8_t* d_q, const int64_t* d_qoff, const uint8_t* d_s,
@@ -131,9 +132,9 @@ public:
                          anyseq_result* out);
     // 2-bit packed DNA batches (batch_packed2.cu)
     int score_batch_packed2_device(const anyseq_scoring& sc, const anyseq_packed_batch& b, int32_t* d_scores,
-                                   anyseq_result* out);
+                                   anyseq_result* out, int32_t* d_ends = nullptr);
     int score_batch_packed2_host(const anyseq_scoring& sc, const anyseq_packed_batch& b, int32_t* scores,
-                                 anyseq_result* out);
+                                 anyseq_result* out, int32_t* ends = nullptr);
     int measure_int_peak(int kind, double* ops_per_s, float* sm_mhz);
     // launch planning without a device (engine.cu); usable on an Engine that was never init()ed
     int plan_launch(int sms, int mode, bool affine, int m, int n, bool chained, const ScoreParams& sp,
@@ -165,7 +166,7 @@ private:
     int plan_bands(int max_h, long long strips_total, int resident, int K, bool chained) const;
     int balance_warps(int nb, int max_h, long long strips_total, int K, bool chained) const;
     int launch_batch(const anyseq_scoring& sc, const ScoreParams& sp, bool affine, BatchArgs& ba, int max_long,
-                     int max_short, cudaStream_t st);
+                     int max_short, int max_q, int max_s, cudaStream_t st);
     // batch.cu: max over pairs of the longer and of the shorter length, optionally of the query and of the subject
     // length and whether some pair has a negative length (synchronises stream_)
     int batch_len_stats(const BatchArgs& ba, int* max_long, int* max_short, int* max_q = nullptr, int* max_s = nullptr,

@@ -223,6 +223,27 @@ int anyseq_score_batch_device(anyseq_ctx* ctx, const anyseq_scoring* sc,
                               const void* d_subjects, const int64_t* d_s_off,
                               int64_t npairs, int32_t* d_scores, anyseq_result* out);
 
+/* Batch scores with end cells: scores[p] as anyseq_score_batch gives it, and ends[2p] / ends[2p+1] = end_i / end_j of
+ * pair p -- what anyseq_score reports for that pair alone (get_score_pos(); local alignment: with the option
+ * "local_end_cell" set), in the caller's coordinates (i: query row, j: subject column):
+ *   global: (lq - 1, ls - 1);
+ *   semiglobal: the last row first (lowest j; j = -1, value 0, wins ties), the last column only if strictly greater
+ *     (lowest i);
+ *   local: the first maximum in row-major order;
+ *   a pair with an empty sequence: (lq - 1, ls - 1).
+ * Local pairs run with the subject as columns, so a local batch whose longest subject exceeds 1024 symbols (512 when
+ * the alphabet needs the generic kernels) gets ANYSEQ_ERR_UNSUPPORTED: score such pairs with anyseq_score and
+ * "local_end_cell".  Everything anyseq_score_batch refuses is refused the same way; ends == NULL is ANYSEQ_ERR_BAD_ARG.
+ * The _device variant takes device pointers for every array. */
+int anyseq_score_batch_ends(anyseq_ctx* ctx, const anyseq_scoring* sc,
+                            const char* queries, const int64_t* q_off,
+                            const char* subjects, const int64_t* s_off,
+                            int64_t npairs, int32_t* scores, int32_t* ends, anyseq_result* out);
+int anyseq_score_batch_ends_device(anyseq_ctx* ctx, const anyseq_scoring* sc,
+                                   const void* d_queries, const int64_t* d_q_off,
+                                   const void* d_subjects, const int64_t* d_s_off,
+                                   int64_t npairs, int32_t* d_scores, int32_t* d_ends, anyseq_result* out);
+
 /* 2-bit packed batches (DNA reads x windows, BASELINE configs[3]; the packed staging of the reference is
  * sequence_to_device, src/mapping_acc.impala:125-131, one byte per symbol).  Four symbols per byte, least significant
  * bits first, A/C/G/T (either case) = 0/1/2/3; every sequence starts on a byte boundary.  Symbols are compared by
@@ -246,6 +267,12 @@ int anyseq_score_batch_packed2(anyseq_ctx* ctx, const anyseq_scoring* sc, const 
                                int32_t* scores, anyseq_result* out);
 int anyseq_score_batch_packed2_device(anyseq_ctx* ctx, const anyseq_scoring* sc, const anyseq_packed_batch* device_batch,
                                       int32_t* d_scores, anyseq_result* out);
+/* The same with end cells (ends[2 * npairs], host resp. device), by the rules of anyseq_score_batch_ends. */
+int anyseq_score_batch_packed2_ends(anyseq_ctx* ctx, const anyseq_scoring* sc, const anyseq_packed_batch* host_batch,
+                                    int32_t* scores, int32_t* ends, anyseq_result* out);
+int anyseq_score_batch_packed2_ends_device(anyseq_ctx* ctx, const anyseq_scoring* sc,
+                                           const anyseq_packed_batch* device_batch, int32_t* d_scores, int32_t* d_ends,
+                                           anyseq_result* out);
 /* Producer-side helper: packs n symbols (A/C/G/T, either case) into ceil(n/4) bytes of out; returns the number of
  * symbols that are not A/C/G/T (they cannot be represented: use the byte path for such sequences). */
 int64_t anyseq_pack2(const char* seq, int64_t n, uint8_t* out);
@@ -275,6 +302,13 @@ typedef struct anyseq_batch_chunk {
 int anyseq_batch_stream_open(anyseq_ctx* ctx, const anyseq_scoring* sc, int64_t cap_pairs,
                              int64_t cap_query_bytes, int64_t cap_subject_bytes, int slots,
                              anyseq_batch_stream** out);
+/* A stream whose chunks also carry end cells (anyseq_score_batch_ends); after collect,
+ * anyseq_batch_stream_chunk_ends gives the chunk's 2 * npairs end cells (pinned, valid until release), and NULL for
+ * a stream opened with anyseq_batch_stream_open. */
+int anyseq_batch_stream_open_ends(anyseq_ctx* ctx, const anyseq_scoring* sc, int64_t cap_pairs,
+                                  int64_t cap_query_bytes, int64_t cap_subject_bytes, int slots,
+                                  anyseq_batch_stream** out);
+const int32_t* anyseq_batch_stream_chunk_ends(anyseq_batch_stream* st, const anyseq_batch_chunk* chunk);
 int anyseq_batch_stream_acquire(anyseq_batch_stream* st, anyseq_batch_chunk* chunk);
 int anyseq_batch_stream_submit(anyseq_batch_stream* st, const anyseq_batch_chunk* chunk);
 int anyseq_batch_stream_finish(anyseq_batch_stream* st);
